@@ -9,6 +9,11 @@ the ranks (all 8 on one GPU at --gpus 1, one per GPU at --gpus 8: strong scaling
 NCCL all-gather of H*(2+Nx) doubles per output reassembles state/covariance.
 
   python bench.py [--gpus N --steps K --warmup W] [--workload c5|c3|c2] [--impl reference]
+                  [--dump-outputs DIR]
+
+--dump-outputs writes the arrays the timed path returned in its last timed step as
+DIR/<name>.npy (float64); the inputs are seeded, so two builds run with the same arguments
+can be compared output for output.
 
 Prints ONE JSON line (rank 0).  `value` = device-resident throughput (CUDA events on the
 engine's stream, max over ranks); `e2e` = the same metric through the host C-ABI call
@@ -30,6 +35,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the source tree
 
 WORKLOADS = {
     'c5': dict(N=16384, Nx=10, Ny=8, H=50, cfg=5, name='C5: N=16384 Nx=10 Ny=8 H=50 TA, outputs sharded over GPUs'),
@@ -59,6 +65,13 @@ def make_workload(N, Nx, Ny, cfg, H):
     A = rt.standard_normal((Nx, Nx))
     Sigma = 1e-4 * np.eye(Nx) + 1e-5 * A @ A.T
     return dict(X=X, Y=Y, hyper=hyper, Z=Z, Sigma=Sigma)
+
+
+def dump_outputs(dirname, **arrays):
+    """--dump-outputs: each array as dirname/<name>.npy in float64."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + '.npy'), np.ascontiguousarray(a, dtype=np.float64))
 
 
 class ClockSampler:
@@ -179,14 +192,16 @@ def run_reference(args, wl, rank):
         mean = np.zeros((H, n_fac)); var = np.zeros((H, n_fac)); J = np.zeros((H, n_fac, Nx))
         for a in range(n_fac):
             mean[:, a], var[:, a], J[:, a] = cpu_predict_port(orc, w['X'], w['hyper'][a], facs[a]['alpha'], facs[a]['chol'], w['Z'])
-        return mean, orc.ta_cov(var, J, w['Sigma'])
+        return dict(mean=mean, var=var, cov=orc.ta_cov(var, J, w['Sigma']), jac=J)
 
     for _ in range(args.warmup):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        out = step()
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, **out)
     t_step = dt * (Ny / n_fac)
     val = H / t_step
     if n_fac == Ny:
@@ -213,7 +228,11 @@ def main():
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--workload', default='c5', choices=sorted(WORKLOADS))
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help="write the last timed step's mean, var, cov and jac to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else max(args.warmup, 1)
     wl = dict(WORKLOADS[args.workload])
     if os.environ.get('GPMPC_BENCH_NY'):          # diagnostics: e.g. one output per GPU on fewer GPUs
@@ -325,6 +344,8 @@ def main():
             e1.record(st)
     eng.synchronize()
     barrier()
+    if args.dump_outputs and rank == 0:       # every rank holds all Ny outputs after the gather
+        dump_outputs(args.dump_outputs, mean=d_mean.cpu(), var=d_var.cpu(), cov=d_cov.cpu(), jac=d_jac.cpu())
     ms_total = sum(e0.elapsed_time(e1) for e0, e1 in evs)
     clocks = sampler.stop()
     tm = torch.tensor([ms_total], dtype=torch.float64, device='cuda')

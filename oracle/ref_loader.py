@@ -14,9 +14,9 @@ and its numpy-only functions run VERBATIM:
     optimize.standardize / normalize (optimize.py:561-587)
 
 Nothing here is copied from the reference; the reference is executed where it
-lies.  ``/root/reference`` does not exist on the GPU box, so this module is only
-used by ``oracle/make_golden.py`` (run here, outputs committed under
-``tests/golden/``) and by CPU tests that skip when the reference is absent.
+lies.  This module is only used by the golden-data generators
+``oracle/make_golden.py`` and ``oracle/make_golden_live.py``, whose outputs are
+committed under ``tests/golden/``; the test-suite never needs the reference.
 """
 from __future__ import annotations
 

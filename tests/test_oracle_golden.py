@@ -1,12 +1,11 @@
 """Pin the CPU oracle: (1) against the reference's own stored model outputs,
 (2) against the committed outputs of the reference's numpy functions run
-verbatim, (3) against the live reference when /root/reference is present,
+verbatim, (3) against a recorded run of the reference at further test points,
 (4) restated CasADi-only parts by finite differences / limiting cases."""
 import numpy as np
 import pytest
 
 from oracle import gp_oracle as orc
-from oracle import ref_loader
 from tests._util import load_fixture, load_golden, relinf
 
 # tolerances: what re-running LAPACK on the stored (X,Y,hyper) reproduces
@@ -58,25 +57,26 @@ def test_matches_reference_numpy_functions_golden(name):
     assert np.all(cv[Ny:] == 0.0)
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason='reference checkout absent')
 @pytest.mark.parametrize('name', ['tank', 'car'])
 def test_matches_live_reference(name):
-    ref = ref_loader.load_reference()
+    """Against a recorded run of the reference's calc_cov_matrix, calc_NLL_numpy and GP.covar
+    at these test points (oracle/make_golden_live.py)."""
+    ref = load_golden('ref_live', name)
     m = load_fixture(name)
     N, Nx = m['X'].shape
     rng = np.random.default_rng(5)
     Zt = m['X'][rng.integers(0, N, 7)] + 0.2 * rng.standard_normal((7, Nx)) * m['X'].std(0)
+    np.testing.assert_array_equal(Zt, ref['Zt'])
     for a in range(m['hyper'].shape[0]):
         ell = m['hyper'][a, :Nx]; sf2 = m['hyper'][a, Nx] ** 2
-        np.testing.assert_allclose(orc.calc_cov_matrix(m['X'], ell, sf2),
-                                   ref.optimize.calc_cov_matrix(m['X'].copy(), ell, sf2), rtol=1e-14)
-        assert orc.calc_NLL(m['hyper'][a], m['X'], m['Y'][:, a]) == pytest.approx(
-            float(ref.optimize.calc_NLL_numpy(m['hyper'][a].copy(), m['X'].copy(), m['Y'][:, a].copy())), rel=1e-13)
-    g = ref_loader.reference_gp_shell(m)
-    np.testing.assert_allclose(orc.covar(m, Zt), g.covar(Zt.copy()), rtol=1e-9, atol=1e-12)
+        K = orc.calc_cov_matrix(m['X'], ell, sf2)
+        np.testing.assert_allclose(K[ref['K_idx']], ref['K_rows'][a], rtol=1e-14)
+        np.testing.assert_allclose(K.sum(1), ref['K_rowsum'][a], rtol=1e-14)
+        assert orc.calc_NLL(m['hyper'][a], m['X'], m['Y'][:, a]) == pytest.approx(ref['nll'][a], rel=1e-13)
+    np.testing.assert_allclose(orc.covar(m, Zt), ref['covar'], rtol=1e-9, atol=1e-12)
     # variance diag of GP.covar == gp_mean_var's var (LU vs triangular solve)
     _, var = orc.gp_mean_var(m['X'], m['hyper'], m['alpha'], m['chol'], Zt)
-    cv = g.covar(Zt.copy())
+    cv = ref['covar']
     for a in range(m['hyper'].shape[0]):
         assert relinf(var[:, a], np.diag(cv[a])) < (1e-8 if name == 'tank' else 5e-6)
 
