@@ -37,6 +37,7 @@ SYMBOLS = [
     ('gpmpc_nlml', C.c_int, [_H, C.c_int, _dp, _dp, _dp]),
     ('gpmpc_predict', C.c_int, [_H, C.c_int, C.c_int, _dp, _dp, C.c_int, _dp, _dp, _dp, _dp]),
     ('gpmpc_predict_grad', C.c_int, [_H, C.c_int, C.c_int, _dp, _dp, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp]),
+    ('gpmpc_predict_hess', C.c_int, [_H, C.c_int, C.c_int, _dp, _dp, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp]),
     ('gpmpc_get_size', C.c_int, [_H, _ip, _ip, _ip]),
     ('gpmpc_append', C.c_int, [_H, _dp, _dp]),
     ('gpmpc_posterior_cov', C.c_int, [_H, C.c_int, _dp, _dp]),
@@ -71,6 +72,15 @@ for _f in ('gp_b200', 'jac_gp_b200'):
     ]
 SYMBOLS += [('gp_b200_bind', C.c_int, [_H, C.c_int, C.c_int]), ('gp_b200_unbind', None, []),
             ('gp_b200_incref', None, []), ('gp_b200_decref', None, [])]
+# the next derivative level of that family: the Jacobian of jac_gp_b200, which CasADi looks up as jac_jac_gp_b200
+_f = 'jac_jac_gp_b200'
+SYMBOLS_HESS = [
+    (_f + '_n_in', _ll, []), (_f + '_n_out', _ll, []),
+    (_f + '_name_in', C.c_char_p, [_ll]), (_f + '_name_out', C.c_char_p, [_ll]),
+    (_f + '_sparsity_in', _llp, [_ll]), (_f + '_sparsity_out', _llp, [_ll]),
+    (_f + '_work', C.c_int, [_llp, _llp, _llp, _llp]),
+    (_f, C.c_int, [_dpp, _dpp, _llp, _dp, C.c_int]),
+]
 
 _lib = None
 
@@ -91,7 +101,7 @@ def load():
             'libgpmpc.so not found at %s -- build it with `python -c "import __graft_entry__ as g; '
             'g.build()"` (nvcc, sm_100a).  This engine has no CPU fallback.' % LIB_PATH)
     lib = C.CDLL(LIB_PATH)
-    for name, res, args in SYMBOLS:
+    for name, res, args in SYMBOLS + SYMBOLS_HESS:
         fn = getattr(lib, name)      # AttributeError if the symbol is missing
         fn.restype = res
         fn.argtypes = args
@@ -265,6 +275,25 @@ class Engine:
         self._check(self.lib.gpmpc_predict_grad(self.h, int(method), H, _ptr(Z), _ptr(Sigma), spp, _ptr(out['mean']),
                                                 _ptr(out['var']), _ptr(out['cov']), _ptr(out['jac']), _ptr(out['dvar_dz']),
                                                 _ptr(out['dcov_dz']), _ptr(out.get('hess'))))
+        return out
+
+    def predict_hess(self, Z, Sigma=None, method=METHOD_TA):
+        """Predict + first and second derivatives w.r.t. the test inputs (gpmpc_predict_hess).
+        Returns the predict_grad dict with hess (H,Ny,Nx,Nx) plus d2var_dz2 (H,Ny,Nx,Nx) and d2cov_dz2 (H,Ny,Ny,Nx,Nx)."""
+        Z = _f64(Z).reshape(-1, self.Nx)
+        H = Z.shape[0]
+        spp = 0
+        if Sigma is not None:
+            Sigma = _f64(Sigma)
+            spp = 1 if Sigma.ndim == 3 else 0
+            assert Sigma.shape == ((H, self.Nx, self.Nx) if spp else (self.Nx, self.Nx))
+        Ny, Nx = self.Ny, self.Nx
+        out = dict(mean=np.empty((H, Ny)), var=np.empty((H, Ny)), cov=np.empty((H, Ny, Ny)), jac=np.empty((H, Ny, Nx)),
+                   dvar_dz=np.empty((H, Ny, Nx)), dcov_dz=np.empty((H, Ny, Ny, Nx)), hess=np.empty((H, Ny, Nx, Nx)),
+                   d2var_dz2=np.empty((H, Ny, Nx, Nx)), d2cov_dz2=np.empty((H, Ny, Ny, Nx, Nx)))
+        self._check(self.lib.gpmpc_predict_hess(self.h, int(method), H, _ptr(Z), _ptr(Sigma), spp,
+                                                *[_ptr(out[k]) for k in ('mean', 'var', 'cov', 'jac', 'dvar_dz', 'dcov_dz',
+                                                                         'hess', 'd2var_dz2', 'd2cov_dz2')]))
         return out
 
     def append(self, x_new, y_new):

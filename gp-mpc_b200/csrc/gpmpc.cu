@@ -84,6 +84,8 @@ struct gpmpc_handle_s {
     double *dCovV = nullptr, *dCovOut = nullptr; long long covVcap = 0, covOutcap = 0;   // GP.covar scratch pool
     // predict_grad: U = Linv^T per output (lazy), beta rows, partial sums, per-batch derivative slabs
     double *dUall = nullptr, *dBeta = nullptr, *dPDV = nullptr, *dPH = nullptr, *dGradOut = nullptr; bool u_valid = false; int gradHcap = 0;
+    // predict_hess: pair-sum partials / sums, Gram of W = L^-1 dks, Sigma Hm scratch, per-batch second-derivative slab
+    double *dHP = nullptr, *dHS = nullptr, *dGram = nullptr, *dSH = nullptr, *dHessOut = nullptr; int hessHcap = 0;
     double *dG = nullptr, *dZ = nullptr, *dSigma = nullptr, *dMean = nullptr, *dVar = nullptr, *dJ = nullptr, *dCov = nullptr;
     double* dRoll = nullptr; size_t rollCap = 0;   // gpmpc_rollout: [Z | Sigma | U | scale | means | vars | cov]
     double *dIn = nullptr, *dOut = nullptr;   // [Z | Sigma] and [mean | var | J | cov] slabs: one H2D + one D2H per host call
@@ -494,7 +496,7 @@ extern "C" int gpmpc_destroy(gpmpc_handle_t h)
     if (h->dCnt) cudaFree(h->dCnt);
     if (h->hPeerStatus) cudaFreeHost(h->hPeerStatus);
     double* bufs[] = {h->dXT, h->dMu, h->dY, h->dHyp, h->dHypTmp, h->dJit, h->dL, h->dLi, h->dW1, h->dW2, h->dAlpha, h->dTmp,
-                      h->dRes, h->dKST, h->dPart, h->dPMJ, h->dSQ, h->dV, h->dR, h->dR2, h->dCovV, h->dCovOut, h->dUall, h->dBeta, h->dPDV, h->dPH, h->dGradOut, h->dG, h->dRoll, h->dIn, h->dOut, h->dU, h->dKinv, h->dGradPart, h->dGrad,
+                      h->dRes, h->dKST, h->dPart, h->dPMJ, h->dSQ, h->dV, h->dR, h->dR2, h->dCovV, h->dCovOut, h->dUall, h->dBeta, h->dPDV, h->dPH, h->dGradOut, h->dHP, h->dHS, h->dGram, h->dSH, h->dHessOut, h->dG, h->dRoll, h->dIn, h->dOut, h->dU, h->dKinv, h->dGradPart, h->dGrad,
                       h->dEmTr, h->dEmLQ, h->dEmVec, h->dEmE2, h->dEmF2, h->dEMP, h->dEmE, h->dEmF, h->dEmW, h->dEmIJ, h->dEmMeanPart, h->dEmPart};
     for (double* b : bufs) if (b) cudaFree(b);
     if (h->dInfo) cudaFree(h->dInfo);
@@ -1440,19 +1442,68 @@ static cudaError_t launch_grad_reduce(gpmpc_handle_t h, const double* dZc, int H
     return cudaGetLastError();
 }
 
-extern "C" int gpmpc_predict_grad(gpmpc_handle_t h, int method, int H, const double* Z, const double* Sigma, int spp,
-                                  double* mean, double* var, double* cov, double* jac,
-                                  double* dvar_dz, double* dcov_dz, double* hess)
+template <int NXP>
+static cudaError_t launch_hess_reduce(gpmpc_handle_t h, const double* dZc, int Hc, int nblk)
+{
+    dim3 g(nblk, Hc, h->nloc);
+    const int smem = (h->Nx * 257 + 512) * 8;
+    static std::atomic<bool> conf[GPMPC_MAX_DEVICES];
+    if (!conf[h->device % GPMPC_MAX_DEVICES].load(std::memory_order_acquire)) {      // dynamic shared memory may pass 48 KB
+        cudaError_t e = cudaFuncSetAttribute(hess_reduce_kernel<NXP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (NX_MAX * 257 + 512) * 8);
+        if (e != cudaSuccess) return e;
+        conf[h->device % GPMPC_MAX_DEVICES].store(true, std::memory_order_release);
+    }
+    hess_reduce_kernel<NXP><<<g, 256, smem, h->st>>>(h->dXT, h->Npad, h->N, h->Nx, h->dHyp, h->Nx + 2, h->dAlpha, h->Npad, dZc,
+                                                      h->dKST, h->dBeta, h->Npad, (long long)HB * h->Npad, h->dHP, nblk, Hc);
+    return cudaGetLastError();
+}
+
+// Second-order work of one chunk of Hc points (after its first-order kernels): W = L^-1 dks on the stream-K product in
+// passes of whole points (floor(HB / Nx) points = up to 64 rows of the A operand, staged in dR; the solved rows land in
+// dV, free once beta is formed), the Gram of each pass, the beta / third-order pair sums, d2var and d2cov.
+static int hess_chunk(gpmpc_handle_t h, int method, int H, int h0, int Hc, const double* dZc, int spp,
+                      const double* d_hess, double* d_d2var, double* d_d2cov)
+{
+    const int np = h->Npad, Nx = h->Nx, Ny = h->Ny;
+    const int nblk_g = (np + GR_CHUNK - 1) / GR_CHUNK;
+    const int ppp = HB / Nx;                                  // points per W pass (NX_MAX = 32 <= HB: at least 2)
+    for (int p0 = 0; p0 < Hc; p0 += ppp) {
+        const int npts = std::min(ppp, Hc - p0), nrows = npts * Nx, bm = (nrows + 7) / 8 * 8;
+        hess_wrows_kernel<<<dim3(np / 128, bm, h->nloc), 128, 0, h->st>>>(h->dXT, np, h->N, Nx, h->dHyp, Nx + 2, dZc,
+                                                                           h->dKST, np, (long long)HB * np, p0, nrows,
+                                                                           h->dR, (long long)HB * np);
+        CUDA_TRY(cudaGetLastError());
+        int rc = tri_product(h, h->dR, h->dLi, bm, nrows, h->dV);
+        if (rc) return rc;
+        hess_gram_kernel<<<dim3(npts, h->nloc), 256, Nx * 129 * 8, h->st>>>(h->dV, np, (long long)HB * np, np, Nx, p0, Hc, h->dGram);
+        CUDA_TRY(cudaGetLastError());
+    }
+    cudaError_t e = (Nx <= 8) ? launch_hess_reduce<8>(h, dZc, Hc, nblk_g)
+                  : (Nx <= 16) ? launch_hess_reduce<16>(h, dZc, Hc, nblk_g) : launch_hess_reduce<32>(h, dZc, Hc, nblk_g);
+    CUDA_TRY(e);
+    hess_finalize_kernel<<<dim3(Hc, h->nloc), 128, 0, h->st>>>(h->dHP, nblk_g, Hc, h->dGram, h->dHyp, Nx + 2, Nx, Ny,
+                                                               h->dG, H, h0, h->dHS, d_d2var);
+    CUDA_TRY(cudaGetLastError());
+    hess_cov_kernel<<<Hc, 256, 3 * Ny * Nx * 8, h->st>>>(Ny, Nx, method == GPMPC_METHOD_TA, h->dSigma, spp, h->dG, H, h0,
+                                                         h->dHyp, Nx + 2, h->dHS, Hc, d_hess, d_d2var, h->dSH, d_d2cov);
+    CUDA_TRY(cudaGetLastError());
+    return GPMPC_OK;
+}
+
+// predict_grad and predict_hess: the first-order outputs of both come from this one sequence of kernels
+static int predict_deriv(gpmpc_handle_t h, const char* fn, int method, int H, const double* Z, const double* Sigma, int spp,
+                         double* mean, double* var, double* cov, double* jac, double* dvar_dz, double* dcov_dz, double* hess,
+                         bool second, double* d2var_dz2, double* d2cov_dz2)
 {
     int rc = predict_check(h, method, H);
     if (rc) return rc;
-    if (method == GPMPC_METHOD_EM) { set_error(h, "gpmpc_predict_grad: derivatives are available for ME and TA"); return GPMPC_ERR_ARG; }
-    if (!Z || (method == GPMPC_METHOD_TA && !Sigma)) { set_error(h, "gpmpc_predict_grad: null Z / Sigma"); return GPMPC_ERR_ARG; }
-    if (h->nloc != h->Ny || h->world != 1) { set_error(h, "gpmpc_predict_grad needs all outputs on one handle (replicate the model, shard the points)"); return GPMPC_ERR_STATE; }
+    if (method == GPMPC_METHOD_EM) { set_error(h, "%s: derivatives are available for ME and TA", fn); return GPMPC_ERR_ARG; }
+    if (!Z || (method == GPMPC_METHOD_TA && !Sigma)) { set_error(h, "%s: null Z / Sigma", fn); return GPMPC_ERR_ARG; }
+    if (h->nloc != h->Ny || h->world != 1) { set_error(h, "%s needs all outputs on one handle (replicate the model, shard the points)", fn); return GPMPC_ERR_STATE; }
     CUDA_TRY(cudaSetDevice(h->device));
     rc = ensure_predict_bufs(h, H);
     if (rc) return rc;
-    NvtxRange nvtx_r("gpmpc.predict_grad");
+    NvtxRange nvtx_r(second ? "gpmpc.predict_hess" : "gpmpc.predict_grad");
     const int np = h->Npad, Nx = h->Nx, Ny = h->Ny, npairs = Nx * (Nx + 1) / 2;
     const int nblk_g = (np + GR_CHUNK - 1) / GR_CHUNK, nblk_mj = (np + ks_chunk(h) - 1) / ks_chunk(h);
     if (!h->dUall) {
@@ -1461,6 +1512,12 @@ extern "C" int gpmpc_predict_grad(gpmpc_handle_t h, int method, int H, const dou
         ALLOC(h->dPDV, (long long)h->nloc * HB * nblk_g * Nx);
         ALLOC(h->dPH, (long long)h->nloc * HB * nblk_g * npairs);
         if (!h->dV) { ALLOC(h->dV, (long long)h->nloc * HB * np); ALLOC(h->dR, (long long)h->nloc * HB * np); }
+    }
+    if (second && !h->dHP) {
+        ALLOC(h->dHP, (long long)h->nloc * HB * nblk_g * npairs * (Nx + 1));
+        ALLOC(h->dHS, (long long)h->nloc * HB * npairs * (Nx + 1));
+        ALLOC(h->dGram, (long long)h->nloc * HB * npairs);
+        ALLOC(h->dSH, (long long)HB * Ny * Nx * Nx);
     }
     if (!h->u_valid) {                 // U = Linv^T (upper): the K-contiguous operand of beta = Linv^T v
         dim3 g(np / 32, np / 32), b(32, 8);
@@ -1478,9 +1535,19 @@ extern "C" int gpmpc_predict_grad(gpmpc_handle_t h, int method, int H, const dou
         ALLOC(h->dGradOut, (long long)std::max(H, HB) * per);
         h->gradHcap = std::max(H, HB);
     }
+    const long long per2 = (long long)Ny * Nx * Nx + (long long)Ny * Ny * Nx * Nx;                  // d2var | d2cov per point
+    if (second && H > h->hessHcap) {
+        CUDA_TRY(cudaStreamSynchronize(h->st));
+        if (h->dHessOut) cudaFree(h->dHessOut);
+        h->dHessOut = nullptr; h->hessHcap = 0;
+        ALLOC(h->dHessOut, (long long)std::max(H, HB) * per2);
+        h->hessHcap = std::max(H, HB);
+    }
     double* d_dvar = h->dGradOut;
     double* d_dcov = d_dvar + (long long)H * Ny * Nx;
     double* d_hess = d_dcov + (long long)H * Ny * Ny * Nx;
+    double* d_d2var = second ? h->dHessOut : nullptr;
+    double* d_d2cov = second ? h->dHessOut + (long long)H * Ny * Nx * Nx : nullptr;
     const size_t nz = (size_t)H * Nx, ns = (method == GPMPC_METHOD_TA) ? (size_t)(spp ? H : 1) * Nx * Nx : 0;
     CUDA_TRY(cudaMemcpyAsync(h->dZ, Z, nz * 8, cudaMemcpyHostToDevice, h->st));
     if (ns) CUDA_TRY(cudaMemcpyAsync(h->dSigma, Sigma, ns * 8, cudaMemcpyHostToDevice, h->st));
@@ -1509,6 +1576,10 @@ extern "C" int gpmpc_predict_grad(gpmpc_handle_t h, int method, int H, const dou
         grad_finalize_kernel<<<dim3(Hc, h->nloc), 128, 0, h->st>>>(h->dPDV, h->dPH, nblk_g, Hc, h->dHyp, Nx + 2, Nx, Ny,
                                                                    h->dG, H, h0, d_dvar, d_hess);
         CUDA_TRY(cudaGetLastError());
+        if (second) {
+            rc = hess_chunk(h, method, H, h0, Hc, dZc, spp, d_hess, d_d2var, d_d2cov);
+            if (rc) return rc;
+        }
     }
     {
         const int smem = (2 * Ny * Nx + Ny) * 8;
@@ -1524,8 +1595,31 @@ extern "C" int gpmpc_predict_grad(gpmpc_handle_t h, int method, int H, const dou
     if (dvar_dz) CUDA_TRY(cudaMemcpyAsync(dvar_dz, d_dvar, (size_t)H * Ny * Nx * 8, cudaMemcpyDeviceToHost, h->st));
     if (dcov_dz) CUDA_TRY(cudaMemcpyAsync(dcov_dz, d_dcov, (size_t)H * Ny * Ny * Nx * 8, cudaMemcpyDeviceToHost, h->st));
     if (hess) CUDA_TRY(cudaMemcpyAsync(hess, d_hess, (size_t)H * Ny * Nx * Nx * 8, cudaMemcpyDeviceToHost, h->st));
+    if (d2var_dz2) CUDA_TRY(cudaMemcpyAsync(d2var_dz2, d_d2var, (size_t)H * Ny * Nx * Nx * 8, cudaMemcpyDeviceToHost, h->st));
+    if (d2cov_dz2) CUDA_TRY(cudaMemcpyAsync(d2cov_dz2, d_d2cov, (size_t)H * Ny * Ny * Nx * Nx * 8, cudaMemcpyDeviceToHost, h->st));
     CUDA_TRY(cudaStreamSynchronize(h->st));
     return GPMPC_OK;
+}
+
+extern "C" int gpmpc_predict_grad(gpmpc_handle_t h, int method, int H, const double* Z, const double* Sigma, int spp,
+                                  double* mean, double* var, double* cov, double* jac,
+                                  double* dvar_dz, double* dcov_dz, double* hess)
+{
+    return predict_deriv(h, "gpmpc_predict_grad", method, H, Z, Sigma, spp, mean, var, cov, jac, dvar_dz, dcov_dz, hess,
+                         false, nullptr, nullptr);
+}
+
+// ------------------------------------------------------------------------------------
+// predict + first and second derivatives w.r.t. the test inputs: everything gpmpc_predict_grad returns plus
+//   d2var_dz2 (H,Ny,Nx,Nx), d2cov_dz2 (H,Ny,Ny,Nx,Nx)   (each optional; formulas above hess_wrows_kernel)
+// ------------------------------------------------------------------------------------
+extern "C" int gpmpc_predict_hess(gpmpc_handle_t h, int method, int H, const double* Z, const double* Sigma, int spp,
+                                  double* mean, double* var, double* cov, double* jac,
+                                  double* dvar_dz, double* dcov_dz, double* hess,
+                                  double* d2var_dz2, double* d2cov_dz2)
+{
+    return predict_deriv(h, "gpmpc_predict_hess", method, H, Z, Sigma, spp, mean, var, cov, jac, dvar_dz, dcov_dz, hess,
+                         true, d2var_dz2, d2cov_dz2);
 }
 
 extern "C" int gpmpc_append(gpmpc_handle_t h, const double* x_new, const double* y_new)

@@ -1792,3 +1792,258 @@ grad_cov_kernel(int Ny, int Nx, int method_ta, const double* __restrict__ Sigma,
         out[idx] = s;
     }
 }
+
+// ---------------------------------------------------------------------------------------
+// Second derivatives of the prediction w.r.t. the test input z (the next level of CasADi's exact
+// Hessian for the MPC's NLP: mpc_class.py:496-513 leaves IPOPT on its default exact Hessian).
+// Per output a and test point z, with s_id = (X_id - z_d)/ell_d^2, beta = K^-1 ks, alpha, J, Hm:
+//   d2var_de = -2 [ w_d^T w_e + sum_i beta_i ks_i s_id s_ie - delta_de (sf2 - var)/ell_d^2 ],
+//              w_d = L^-1 (ks o s_.d)                     (beta^T ks = sum v^2 = sf2 - var)
+//   T_fde    = d^3 mean / dz_f dz_d dz_e
+//            = sum_i alpha_i ks_i s_if s_id s_ie - delta_fd J_e/ell_f^2 - delta_fe J_d/ell_f^2 - delta_de J_f/ell_d^2
+//   'TA' d2cov_ab,de = delta_ab d2var_a,de + sum_f [ T_a,fde (Sigma J_b)_f + Hm_a,fd (Sigma Hm_b)_fe
+//                                                + Hm_a,fe (Sigma Hm_b)_fd + (J_a Sigma)_f T_b,fde ]
+//   'ME' d2cov_ab,de = delta_ab d2var_a,de
+// Pairs (d <= e) are packed row-major: q = d*Nx - d(d-1)/2 + (e - d).
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ void pair_de(int q, int Nx, int& d, int& e)
+{
+    int base = 0;
+    d = 0;
+    while (base + (Nx - d) <= q) { base += Nx - d; ++d; }
+    e = d + (q - base);
+}
+__device__ __forceinline__ int pair_q(int d, int e, int Nx) { return d * Nx - d * (d - 1) / 2 + (e - d); }
+
+// A operand of the W = L^-1 dks product: row r = pl*Nx + d holds ks_i s_id of chunk point p0 + pl (columns i < N;
+// the padding columns and the rows r >= nrows up to the fragment height are zero).  grid (Npad/128, bm, outputs).
+__global__ void __launch_bounds__(128)
+hess_wrows_kernel(const double* __restrict__ XT, int ldx, int N, int Nx,
+                  const double* __restrict__ hyp, int hyp_ld, const double* __restrict__ Z,
+                  const double* __restrict__ KST, int ldk, long long sK, int p0, int nrows,
+                  double* __restrict__ A, long long sA)
+{
+    const int i = blockIdx.x * 128 + threadIdx.x, r = blockIdx.y, a = blockIdx.z;
+    double v = 0.0;
+    if (r < nrows && i < N) {
+        const int pl = r / Nx, d = r - pl * Nx, hl = p0 + pl;
+        const double e = hyp[(long long)a * hyp_ld + d];
+        const double sd = (XT[(long long)d * ldx + i] - Z[(long long)hl * Nx + d]) * (1.0 / (e * e));
+        v = KST[(long long)a * sK + (long long)hl * ldk + i] * sd;
+    }
+    A[(long long)a * sA + (long long)r * ldk + i] = v;
+}
+
+// Gram step: GRAM[a][p0+pl][q(d<=e)] = w_d^T w_e over the Npad columns of the solved rows pl*Nx + d.
+// grid (points of the pass, outputs), 256 threads; columns staged 128 at a time.
+__global__ void __launch_bounds__(256)
+hess_gram_kernel(const double* __restrict__ W, int ldw, long long sW, int np, int Nx, int p0, int Hc,
+                 double* __restrict__ GRAM)
+{
+    extern __shared__ double gsm[];                 // S[Nx][129]
+    const int pl = blockIdx.x, a = blockIdx.y, tid = threadIdx.x;
+    const int npairs = Nx * (Nx + 1) / 2;
+    const double* Wp = W + (long long)a * sW + (long long)pl * Nx * ldw;
+    double acc[3] = {0.0, 0.0, 0.0};                // pairs tid, tid+256, tid+512 (NX_MAX = 32: 528 pairs)
+    for (int c0 = 0; c0 < np; c0 += 128) {
+        for (int idx = tid; idx < Nx * 128; idx += 256) {
+            const int d = idx >> 7, t = idx & 127;
+            gsm[d * 129 + t] = Wp[(long long)d * ldw + c0 + t];
+        }
+        __syncthreads();
+#pragma unroll
+        for (int r = 0; r < 3; ++r) {
+            const int q = tid + 256 * r;
+            if (q < npairs) {
+                int d, e;
+                pair_de(q, Nx, d, e);
+                const double* sd = gsm + d * 129; const double* se = gsm + e * 129;
+                double s = 0.0;
+                for (int t = 0; t < 128; ++t) s = fma(sd[t], se[t], s);
+                acc[r] += s;
+            }
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        const int q = tid + 256 * r;
+        if (q < npairs) GRAM[((long long)a * Hc + p0 + pl) * npairs + q] = acc[r];
+    }
+}
+
+// Per (output, test point, GR_CHUNK-point block): for every pair q = (d <= e), the (pairs x N).(N x (1+Nx)) product
+//   HP[q][0] = sum_i beta_i ks_i s_id s_ie          HP[q][1+f] = sum_i alpha_i ks_i s_id s_ie s_if
+// A thread owns whole pairs; its 1 + Nx sums live in registers over one 256-point sub-block and in its own slice of
+// the block's partial record between sub-blocks (no other thread touches it).  grid (Npad/GR_CHUNK, Hc, outputs).
+template <int NXP>
+__global__ void __launch_bounds__(256)
+hess_reduce_kernel(const double* __restrict__ XT, int ldx, int N, int Nx,
+                   const double* __restrict__ hyp, int hyp_ld,
+                   const double* __restrict__ alpha, long long sal,
+                   const double* __restrict__ Z,
+                   const double* __restrict__ KST, const double* __restrict__ BETA, int ldk, long long sK,
+                   double* __restrict__ HP, int nblk, int Hc)
+{
+    extern __shared__ double hsm[];                 // S[Nx][257], WA[256], WB[256]
+    __shared__ double zs[NXP], ie2[NXP];
+    const int a = blockIdx.z, h = blockIdx.y, blk = blockIdx.x, tid = threadIdx.x;
+    double* S = hsm; double* WA = hsm + Nx * 257; double* WB = WA + 256;
+    const double* hp = hyp + (long long)a * hyp_ld;
+    if (tid < NXP) {
+        const double e = (tid < Nx) ? hp[tid] : 1.0;
+        zs[tid] = (tid < Nx) ? Z[(long long)h * Nx + tid] : 0.0;
+        ie2[tid] = 1.0 / (e * e);
+    }
+    __syncthreads();
+    const int npairs = Nx * (Nx + 1) / 2, F1 = Nx + 1;
+    const double* ks = KST + (long long)a * sK + (long long)h * ldk;
+    const double* be = BETA + (long long)a * sK + (long long)h * ldk;
+    const double* al = alpha + (long long)a * sal;
+    double* out = HP + (((long long)a * Hc + h) * nblk + blk) * npairs * F1;
+    for (int sub = 0; sub < GR_CHUNK / 256; ++sub) {
+        const int i = blk * GR_CHUNK + sub * 256 + tid;
+        double k = 0.0, wa = 0.0, wb = 0.0;
+        if (i < N) { k = ks[i]; wa = al[i] * k; wb = be[i] * k; }
+        for (int d = 0; d < Nx; ++d)
+            S[d * 257 + tid] = (i < N) ? (XT[(long long)d * ldx + i] - zs[d]) * ie2[d] : 0.0;
+        WA[tid] = wa; WB[tid] = wb;
+        __syncthreads();
+        for (int q = tid; q < npairs; q += 256) {
+            int d, e;
+            pair_de(q, Nx, d, e);
+            double* o = out + (long long)q * F1;
+            double accb = (sub == 0) ? 0.0 : o[0];
+            double acc[NXP];
+#pragma unroll
+            for (int f = 0; f < NXP; ++f) acc[f] = (sub == 0 || f >= Nx) ? 0.0 : o[1 + f];
+            const double* sd = S + d * 257; const double* se = S + e * 257;
+            for (int t = 0; t < 256; ++t) {
+                const double pde = sd[t] * se[t];
+                accb = fma(WB[t], pde, accb);
+                const double pa = WA[t] * pde;
+#pragma unroll
+                for (int f = 0; f < NXP; ++f)
+                    if (f < Nx) acc[f] = fma(pa, S[f * 257 + t], acc[f]);
+            }
+            o[0] = accb;
+#pragma unroll
+            for (int f = 0; f < NXP; ++f)
+                if (f < Nx) o[1 + f] = acc[f];
+        }
+        __syncthreads();
+    }
+}
+
+// Per (chunk point h, output a): the block partials summed in block order into HS[a][h][q][1+Nx], and
+// d2var (H,Ny,Nx,Nx) from the Gram, the beta pair sums and var of the gather record; (d,e) and (e,d) get one value.
+// grid (Hc, outputs), 128 threads.
+__global__ void __launch_bounds__(128)
+hess_finalize_kernel(const double* __restrict__ HP, int nblk, int Hc, const double* __restrict__ GRAM,
+                     const double* __restrict__ hyp, int hyp_ld, int Nx, int Ny,
+                     const double* __restrict__ G, int Htot, int h0,
+                     double* __restrict__ HS, double* __restrict__ d2var)
+{
+    const int h = blockIdx.x, a = blockIdx.y, tid = threadIdx.x;
+    const int npairs = Nx * (Nx + 1) / 2, nent = npairs * (Nx + 1);
+    const long long rec = (long long)a * Hc + h;
+    const double* src = HP + rec * nblk * nent;
+    double* dst = HS + rec * nent;
+    for (int k = tid; k < nent; k += 128) {
+        double s = 0.0;
+        for (int b = 0; b < nblk; ++b) s += src[(long long)b * nent + k];
+        dst[k] = s;
+    }
+    const double* hp = hyp + (long long)a * hyp_ld;
+    const double sf = hp[Nx];
+    const double c = sf * sf - G[(((long long)a) * Htot + h0 + h) * (Nx + 2) + 1];      // beta^T ks = sf2 - var
+    double* out = d2var + (((long long)(h0 + h)) * Ny + a) * Nx * Nx;
+    for (int q = tid; q < npairs; q += 128) {
+        int d, e;
+        pair_de(q, Nx, d, e);
+        double pb = 0.0;
+        for (int b = 0; b < nblk; ++b) pb += src[(long long)b * nent + (long long)q * (Nx + 1)];
+        double v = GRAM[rec * npairs + q] + pb;
+        if (d == e) v -= c / (hp[d] * hp[d]);
+        v *= -2.0;
+        out[d * Nx + e] = v;
+        out[e * Nx + d] = v;
+    }
+}
+
+// T_fde of output a at chunk point h from the summed third-order sums (see the block comment above)
+__device__ __forceinline__ double hess_T(const double* HSa, const double* Ja, const double* hp, int Nx, int f, int d, int e)
+{
+    double t = HSa[(long long)pair_q(min(d, e), max(d, e), Nx) * (Nx + 1) + 1 + f];
+    if (f == d) t -= Ja[e] / (hp[f] * hp[f]);
+    if (f == e) t -= Ja[d] / (hp[f] * hp[f]);
+    if (d == e) t -= Ja[f] / (hp[d] * hp[d]);
+    return t;
+}
+
+// d2cov (H,Ny,Ny,Nx,Nx) of the chunk's points: grid (Hc), 256 threads.  J comes from the gather records, Hm from
+// grad_finalize_kernel; SH[b][f][e] = (Sigma Hm_b)[f][e] is staged in global scratch (Ny Nx^2 per point).
+__global__ void __launch_bounds__(256)
+hess_cov_kernel(int Ny, int Nx, int method_ta, const double* __restrict__ Sigma, int sigma_per_point,
+                const double* __restrict__ G, int Htot, int h0, const double* __restrict__ hyp, int hyp_ld,
+                const double* __restrict__ HS, int Hc, const double* __restrict__ hess,
+                const double* __restrict__ d2var, double* __restrict__ SH, double* __restrict__ d2cov)
+{
+    extern __shared__ double csm[];                 // Jh[Ny][Nx], SJ[Ny][Nx] = Sigma J_b, JS[Ny][Nx] = J_a Sigma
+    double* Jh = csm; double* SJ = csm + Ny * Nx; double* JS = csm + 2 * Ny * Nx;
+    const int h = blockIdx.x, hg = h0 + h, tid = threadIdx.x;
+    const int nxx = Nx * Nx;
+    const double* dv = d2var + (long long)hg * Ny * nxx;
+    double* out = d2cov + (long long)hg * Ny * Ny * nxx;
+    if (!method_ta) {
+        for (long long idx = tid; idx < (long long)Ny * Ny * nxx; idx += 256) {
+            const int de = (int)(idx % nxx), b = (int)((idx / nxx) % Ny), a = (int)(idx / ((long long)nxx * Ny));
+            out[idx] = (a == b) ? dv[(long long)a * nxx + de] : 0.0;
+        }
+        return;
+    }
+    for (int idx = tid; idx < Ny * Nx; idx += 256) {
+        const int a = idx / Nx, d = idx - a * Nx;
+        Jh[idx] = G[(((long long)a) * Htot + hg) * (Nx + 2) + 2 + d];
+    }
+    __syncthreads();
+    const double* Sg = Sigma + (sigma_per_point ? (long long)hg * nxx : 0);
+    const double* Hh = hess + (long long)hg * Ny * nxx;
+    double* SHh = SH + (long long)h * Ny * nxx;
+    for (int idx = tid; idx < Ny * Nx; idx += 256) {
+        const int a = idx / Nx, d = idx - a * Nx;
+        double s1 = 0.0, s2 = 0.0;
+        for (int e = 0; e < Nx; ++e) {
+            s1 = fma(Sg[d * Nx + e], Jh[a * Nx + e], s1);          // (Sigma J_a)[d]
+            s2 = fma(Jh[a * Nx + e], Sg[e * Nx + d], s2);          // (J_a Sigma)[d]
+        }
+        SJ[idx] = s1; JS[idx] = s2;
+    }
+    for (int idx = tid; idx < Ny * nxx; idx += 256) {
+        const int b = idx / nxx, f = (idx / Nx) % Nx, e = idx % Nx;
+        const double* Hb = Hh + (long long)b * nxx;
+        double s = 0.0;
+        for (int g = 0; g < Nx; ++g) s = fma(Sg[f * Nx + g], Hb[g * Nx + e], s);
+        SHh[idx] = s;
+    }
+    __syncthreads();
+    const int npairs = Nx * (Nx + 1) / 2, nent = npairs * (Nx + 1);
+    for (int idx = tid; idx < Ny * Ny * npairs; idx += 256) {
+        const int q = idx % npairs, b = (idx / npairs) % Ny, a = idx / (npairs * Ny);
+        int d, e;
+        pair_de(q, Nx, d, e);
+        const double* hpa = hyp + (long long)a * hyp_ld; const double* hpb = hyp + (long long)b * hyp_ld;
+        const double* HSa = HS + ((long long)a * Hc + h) * nent; const double* HSb = HS + ((long long)b * Hc + h) * nent;
+        const double* Ha = Hh + (long long)a * nxx; const double* SHb = SHh + (long long)b * nxx;
+        double s = (a == b) ? dv[(long long)a * nxx + d * Nx + e] : 0.0;
+        for (int f = 0; f < Nx; ++f) {
+            s = fma(hess_T(HSa, Jh + a * Nx, hpa, Nx, f, d, e), SJ[b * Nx + f], s);
+            s = fma(Ha[f * Nx + d], SHb[f * Nx + e], s);
+            s = fma(Ha[f * Nx + e], SHb[f * Nx + d], s);
+            s = fma(JS[a * Nx + f], hess_T(HSb, Jh + b * Nx, hpb, Nx, f, d, e), s);
+        }
+        double* o = out + ((long long)a * Ny + b) * nxx;
+        o[d * Nx + e] = s;
+        o[e * Nx + d] = s;
+    }
+}

@@ -372,6 +372,41 @@ class GP:
         out.update(mean=mean, dmean_dz=jac, dcov_dz=dcov)
         return out
 
+    def predict_batch_hess(self, x, u, cov=None, method=None):
+        """Second-order companion of predict_batch_grad: what IPOPT's exact Hessian (the reference's nlpsol setup,
+        mpc_class.py:496-513) needs from the GP.  Returns predict_batch_grad's dict plus
+            d2mean_dz2 (H,Ny,Nx,Nx)          d^2 mean / d z_d d z_e in the caller's units
+            d2cov_dz2  (H,Ny,Ny,Nx,Nx)       d^2 cov / d z_d d z_e (cov itself is not rescaled: only 1/stdZ enters)
+            d2cov_dzdSigma_factor (H,Ny,Nx,Nx)  Hm with d^2 cov[a][b] / d z_d d Sigma[f][g] =
+                                             Hm[a][f][d] J[b][g] + J[a][f] Hm[b][g][d],  J = dcov_dSigma_factor
+        Methods 'ME' and 'TA'; all outputs on one GPU."""
+        method = method or self.__gp_method
+        if method not in ('ME', 'TA'):
+            raise NotImplementedError("derivatives are available for gp_method 'ME' and 'TA'")
+        if self.__comm.world > 1 and self.__mode == 'outputs':
+            raise NotImplementedError('predict_batch_hess needs all outputs on one GPU (build the GP with a single-process Comm)')
+        x = np.asarray(x, dtype=np.float64).reshape(-1, self.__Ny)
+        u = np.asarray(u, dtype=np.float64).reshape(x.shape[0], self.__Nu)
+        if self.__normalize:
+            x = self.standardize(x, self.__meanX, self.__stdX)
+            u = self.standardize(u, self.__meanU, self.__stdU)
+        Z = np.hstack([x, u])
+        if cov is None and method == 'TA':
+            cov = np.zeros((self.__Nx, self.__Nx))
+        g = self.__engine.predict_hess(Z, cov if method == 'TA' else None, _GPU_METHODS[method])
+        mean, jac, dcov, hess, d2cov = g['mean'], g['jac'], g['dcov_dz'], g['hess'], g['d2cov_dz2']
+        out = dict(cov=g['cov'], dcov_dSigma_factor=jac.copy(), d2cov_dzdSigma_factor=hess.copy())
+        if self.__normalize:
+            sz = self.__stdZ
+            mean = self.inverse_mean(mean, self.__meanY, self.__stdY)
+            jac = jac * self.__stdY[None, :, None] / sz[None, None, :]
+            dcov = dcov / sz[None, None, None, :]
+            hess = hess * self.__stdY[None, :, None, None] / (sz[:, None] * sz[None, :])[None, None]
+            d2cov = d2cov / (sz[:, None] * sz[None, :])[None, None, None]
+            out['d2cov_dzdSigma_factor'] = out['d2cov_dzdSigma_factor'] / sz[None, None, None, :]
+        out.update(mean=mean, dmean_dz=jac, dcov_dz=dcov, d2mean_dz2=hess, d2cov_dz2=d2cov)
+        return out
+
     def predict(self, x, u, cov):
         """ Predict future state  (reference gp_class.py:245-263)
 

@@ -142,6 +142,19 @@ int gpmpc_predict_grad(gpmpc_handle_t h, int method, int H, const double* Z, con
                        int sigma_per_point, double* mean, double* var, double* cov, double* jac,
                        double* dvar_dz, double* dcov_dz, double* hess);
 
+/* Prediction plus its first AND second derivatives w.r.t. the test inputs -- what IPOPT's default exact Hessian
+ * needs from the GP when nlpsol builds the MPC's NLP with 'expand': True and no hessian_approximation
+ * (mpc_class.py:496-513; CasADi differentiates the symbolic build_gp / build_TA_cov graphs of gp_functions.py:111-173
+ * twice).  Same arguments and outputs as gpmpc_predict_grad (equal to them bit for bit), plus, each optional:
+ *   d2var_dz2 (H,Ny,Nx,Nx)     d^2 var_a / d z_d d z_e          (one extra L^-1 product with H*Nx rows per output)
+ *   d2cov_dz2 (H,Ny,Ny,Nx,Nx)  d^2 cov[a][b] / d z_d d z_e of diag(var) ('ME') or diag(var) + J Sigma J^T ('TA')
+ * Both are exactly symmetric in (d, e).  The mixed block d^2 cov[a][b] / d z_d d Sigma[f][g] =
+ * hess_a[f][d] J_b[g] + J_a[f] hess_b[g][d] is formed by the caller from jac and hess; the Sigma-Sigma block is 0.
+ * Methods ME and TA; the handle must own all outputs (GPMPC_ERR_STATE otherwise). */
+int gpmpc_predict_hess(gpmpc_handle_t h, int method, int H, const double* Z, const double* Sigma,
+                       int sigma_per_point, double* mean, double* var, double* cov, double* jac,
+                       double* dvar_dz, double* dcov_dz, double* hess, double* d2var_dz2, double* d2cov_dz2);
+
 /* Open-loop multi-step prediction with the state kept on the device: the numeric loop of GP.predict_compare
  * (gp_class.py:746-804, :779-792: mean_t, covar_x = predict(mean_t, u_t, covar); covar[:Ny,:Ny] = covar_x) for a
  * model whose inputs are z = [x, u] (Nx = Ny + Nu).  All Nt steps are enqueued back to back, one synchronisation.

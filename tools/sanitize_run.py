@@ -1,7 +1,7 @@
 """Small end-to-end pass over every kernel of the engine for compute-sanitizer
 (memcheck / racecheck / synccheck / initcheck):  K build, leaf + DMMA GEMMs (cp.async and TMA
 tensor-map feeds), alpha, NLML + gradient, the persistent stream-K predict kernel with tile
-fix-ups (several grid sizes, lower and upper mode), predict_grad, EM, rank-1 append, GP.covar.
+fix-ups (several grid sizes, lower and upper mode), predict_grad, predict_hess (W passes, pair sums), EM, rank-1 append, GP.covar.
     compute-sanitizer --tool racecheck python tools/sanitize_run.py"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -28,6 +28,11 @@ eng.set_option('predict_ctas', 5)
 g = eng.predict_grad(p['Z'], p['Sigma'], L.METHOD_TA, want_hess=True)
 fd = orc.predict_grad_fd(p['X'], p['hyper'], post['alpha'], post['chol'], p['Z'], p['Sigma'], 'TA')
 print('grad', relinf(g['dvar_dz'], fd['dvar']), relinf(g['dcov_dz'], fd['dcov']), flush=True)
+from tests._hess_oracle import predict_hess_closed
+for meth, name, S in ((L.METHOD_TA, 'TA', p['Sigma']), (L.METHOD_ME, 'ME', None)):
+    g2 = eng.predict_hess(p['Z'], S, meth)
+    c2 = predict_hess_closed(p['X'], p['hyper'], post['alpha'], post['chol'], p['Z'], p['Sigma'], name)
+    print('hess', name, relinf(g2['d2var_dz2'], c2['d2var']), relinf(g2['d2cov_dz2'], c2['d2cov']), flush=True)
 eng.set_option('refine', 1)
 mean, var, _, _ = eng.predict(p['Z'], p['Sigma'], L.METHOD_TA)
 print('refine', relinf(var, vo), flush=True)
