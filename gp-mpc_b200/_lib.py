@@ -34,6 +34,8 @@ SYMBOLS = [
     ('gpmpc_set_y', C.c_int, [_H, C.c_int, _dp]),
     ('gpmpc_build_K', C.c_int, [_H, C.c_int, _dp]),
     ('gpmpc_factorize', C.c_int, [_H, C.c_double, _ip]),
+    ('gpmpc_fitc', C.c_int, [_H, C.c_int, _dp, _dp, C.c_double, _ip, _dp]),
+    ('gpmpc_fitc_timings', C.c_int, [_H, _dp]),
     ('gpmpc_nlml', C.c_int, [_H, C.c_int, _dp, _dp, _dp]),
     ('gpmpc_predict', C.c_int, [_H, C.c_int, C.c_int, _dp, _dp, C.c_int, _dp, _dp, _dp, _dp]),
     ('gpmpc_predict_grad', C.c_int, [_H, C.c_int, C.c_int, _dp, _dp, C.c_int, _dp, _dp, _dp, _dp, _dp, _dp, _dp]),
@@ -184,6 +186,27 @@ class Engine:
             raise np.linalg.LinAlgError(self.lib.gpmpc_last_error(self.h).decode())
         self._check(rc)
         return info
+
+    def fitc(self, X, Y, jitter=1e-6):
+        """FITC sparse model (gpmpc_fitc): the handle's own points are the M inducing points, X:(N,Nx), Y:(N,Ny) the
+        training set in the GP's input space.  Returns (info, nll) per owned output: info 1 = the B factor needed its
+        retry shift, nll = FITC negative log marginal likelihood.  Afterwards every predict method evaluates FITC."""
+        X = _f64(X); Y = _f64(Y)
+        N = X.shape[0]
+        X = X.reshape(N, self.Nx); Y = Y.reshape(N, self.Ny)
+        info = np.zeros(self.out_count, dtype=np.int32)
+        nll = np.zeros(self.out_count)
+        rc = self.lib.gpmpc_fitc(self.h, int(N), _ptr(X), _ptr(Y), float(jitter), info.ctypes.data_as(_ip), _ptr(nll))
+        if rc == ERR_NOTPD:
+            raise np.linalg.LinAlgError(self.lib.gpmpc_last_error(self.h).decode())
+        self._check(rc)
+        return info, nll
+
+    def fitc_timings(self):
+        """Phase times (ms) of the last fitc build: dict(kuf, v_product, column_pass, syrk, factorisations)."""
+        out = np.zeros(5)
+        self._check(self.lib.gpmpc_fitc_timings(self.h, _ptr(out)))
+        return dict(zip(('kuf', 'v_product', 'column_pass', 'syrk', 'factorisations'), out))
 
     def nlml(self, a, theta, grad=True):
         theta = _f64(theta, (self.Nx + 2,))

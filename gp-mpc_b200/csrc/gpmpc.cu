@@ -101,6 +101,9 @@ struct gpmpc_handle_s {
     std::vector<double> hyper;        // (nloc, Nx+2)
     std::vector<double> logdet, yalpha;
     std::vector<int> jitter_used;
+    // FITC sparse model (gpmpc_fitc): L holds Luu, Li holds R (R^T R = K~^-1), alpha holds alpha_s
+    bool sparse = false; int opt_fitc_panel = 4096;
+    double fitc_ms[5] = {0, 0, 0, 0, 0};   // last build: Kuf, V product, column pass + b, SYRK, M-sized factorisations
     int opt_refine = 0, opt_gemm_variant = 3, opt_leaf_variant = 3, opt_small_tiles = 592;   // 128x64-tile count below which 64x32 tiles are used
     // comm
     nccl_comm_t comm = nullptr; int rank = 0, world = 1;
@@ -668,7 +671,7 @@ extern "C" int gpmpc_factorize(gpmpc_handle_t h, double jitter, int* info)
     CUDA_TRY(cudaMemcpyAsync(res.data(), h->dRes, 2 * nl * 8, cudaMemcpyDeviceToHost, h->st));
     CUDA_TRY(cudaStreamSynchronize(h->st));
     for (int a = 0; a < nl; ++a) { h->logdet[a] = res[2 * a]; h->yalpha[a] = res[2 * a + 1]; }
-    h->factorized = true; h->u_valid = false;
+    h->factorized = true; h->u_valid = false; h->sparse = false;
     return GPMPC_OK;
 }
 
@@ -687,6 +690,234 @@ static int compute_kinv(gpmpc_handle_t h, int al)
     p.mt = np / 128; p.nt = np / 128; p.K = np; p.alpha = 1.0; p.beta = 0.0;
     p.kflags = GEMM_KI_GE | GEMM_KJ_GE; p.lower = 1;
     CUDA_TRY(gemm128(h, true, p, 1));
+    return GPMPC_OK;
+}
+
+// ------------------------------------------------------------------------------------
+// FITC sparse model (the reference's GP.sparse, gp_class.py:682-689).  The handle's own M points are the inducing points;
+// the N training points stream through the GPU in column panels of opt_fitc_panel points:
+//   Luu = chol(Kuu + jitter sf2 I),  V = Luu^-1 Kuf,  Lambda = diag(Kff - V^T V) + sn2 I,  A = I + V Lambda^-1 V^T = LA LA^T
+//   B = I - A^-1 = Luu^T K~^-1 Luu,  S^T S = B (reverse Cholesky),  R = S Luu^-1,  alpha_s = Luu^-T LA^-T LA^-1 V Lambda^-1 y
+// R goes to the L^-1 slab and alpha_s to alpha, so every predict kernel evaluates the FITC predictive distribution.
+// ------------------------------------------------------------------------------------
+#define FITC_N_MAX (1 << 30)          // panel column indices and the padded column count stay in int
+#define FITC_B_SHIFT 1e-10            // retry shift of B: moves the variance by at most FITC_B_SHIFT * Qss <= 1e-10 sf2
+
+// build buffers: allocated per call, freed on every return path (only L, L^-1 and alpha outlive the build)
+struct FitcBufs {
+    gpmpc_handle_t h;
+    double *X = nullptr, *Y = nullptr, *Kuf = nullptr, *V = nullptr, *P[4] = {nullptr, nullptr, nullptr, nullptr};
+    double *b = nullptr, *t = nullptr, *w = nullptr, *part = nullptr, *res = nullptr, *hyp = nullptr;
+    std::vector<cudaEvent_t> ev;        // phase boundaries: [Kuu start, Kuu end, 4 per panel..., panels end, build end]
+    explicit FitcBufs(gpmpc_handle_t hh) : h(hh) {}
+    ~FitcBufs()
+    {
+        cudaStreamSynchronize(h->st);
+        for (cudaEvent_t e : ev) cudaEventDestroy(e);
+        double* bufs[] = {X, Y, Kuf, V, P[0], P[1], P[2], P[3], b, t, w, part, res, hyp};
+        for (double* q : bufs) if (q) cudaFree(q);
+    }
+};
+
+static int fitc_check_info(gpmpc_handle_t h, const char* what, std::vector<int>& inf)
+{
+    CUDA_TRY(cudaMemcpyAsync(inf.data(), h->dInfo, inf.size() * sizeof(int), cudaMemcpyDeviceToHost, h->st));
+    CUDA_TRY(cudaStreamSynchronize(h->st));
+    for (size_t a = 0; a < inf.size(); ++a)
+        if (inf[a]) {
+            set_error(h, "gpmpc_fitc: output %d: %s is not positive definite (pivot %d)", h->a0 + (int)a, what, inf[a] - 1);
+            return GPMPC_ERR_NOTPD;
+        }
+    return GPMPC_OK;
+}
+
+extern "C" int gpmpc_fitc(gpmpc_handle_t h, int N, const double* X, const double* Y, double jitter, int* info, double* nll)
+{
+    if (!h) return GPMPC_ERR_ARG;
+    if (!X || !Y || N < 1 || N > FITC_N_MAX || !(jitter >= 0.0)) {
+        set_error(h, "gpmpc_fitc: need X, Y, 1 <= N <= %d (got %d) and jitter >= 0", FITC_N_MAX, N);
+        return GPMPC_ERR_ARG;
+    }
+    if (!h->has_data || !h->has_hyper) { set_error(h, "gpmpc_fitc: set_data (the inducing points) and set_hyper first"); return GPMPC_ERR_STATE; }
+    if (h->opt_refine) { set_error(h, "gpmpc_fitc: option refine needs the dense factor; switch it off first"); return GPMPC_ERR_STATE; }
+    const int nl = h->nloc, Nx = h->Nx, M = h->N, mp = h->Npad, m = Nx + 2;
+    for (int a = 0; a < nl; ++a)
+        if (!(h->hyper[(size_t)a * m + Nx + 1] != 0.0)) { set_error(h, "gpmpc_fitc: output %d has sn = 0 (FITC needs noise)", h->a0 + a); return GPMPC_ERR_ARG; }
+    CUDA_TRY(cudaSetDevice(h->device));
+    NvtxRange nvtx_r("gpmpc.fitc");
+    h->factorized = false; h->sparse = false; h->u_valid = false;
+    const int nb = h->opt_fitc_panel, npan = (int)(((long long)N + nb - 1) / nb), cpp = nb / 32;
+    const long long Nq = (long long)npan * nb, sK = (long long)mp * nb, sP = slab(h), nparts = (long long)npan * cpp;
+    FitcBufs f(h);
+    ALLOC(f.X, (long long)Nx * Nq); ALLOC(f.Y, (long long)nl * Nq);
+    ALLOC(f.Kuf, nl * sK); ALLOC(f.V, nl * sK);
+    for (int k = 0; k < 4; ++k) ALLOC(f.P[k], nl * sP);
+    ALLOC(f.b, (long long)nl * mp); ALLOC(f.t, 2LL * nl * mp); ALLOC(f.w, (long long)nl * nb);
+    ALLOC(f.part, 2 * nl * nparts); ALLOC(f.res, nl); ALLOC(f.hyp, (long long)nl * m);
+    {   // training set, transposed (X^T: Nx x Nq) and per owned output (Y: nl x Nq), zero padded to whole panels
+        std::vector<double> xt((size_t)Nx * Nq, 0.0), yl((size_t)nl * Nq, 0.0);
+        for (long long i = 0; i < N; ++i)
+            for (int d = 0; d < Nx; ++d) xt[(size_t)d * Nq + i] = X[(size_t)i * Nx + d];
+        for (int a = 0; a < nl; ++a)
+            for (long long i = 0; i < N; ++i) yl[(size_t)a * Nq + i] = Y[(size_t)i * h->Ny + h->a0 + a];
+        CUDA_TRY(cudaMemcpyAsync(f.X, xt.data(), xt.size() * 8, cudaMemcpyHostToDevice, h->st));
+        CUDA_TRY(cudaMemcpyAsync(f.Y, yl.data(), yl.size() * 8, cudaMemcpyHostToDevice, h->st));
+        CUDA_TRY(cudaStreamSynchronize(h->st));
+    }
+    f.ev.assign(4 * npan + 4, nullptr);
+    for (auto& e : f.ev) CUDA_TRY(cudaEventCreate(&e));
+    std::vector<int> inf(nl, 0);
+    // 1. Kuu + jitter sf2 I (the K build with sn = 0) -> Luu (L slab), Luu^-1 (P0)
+    {
+        std::vector<double> hk(h->hyper), jit(nl);
+        for (int a = 0; a < nl; ++a) {
+            const double sf = hk[(size_t)a * m + Nx];
+            hk[(size_t)a * m + Nx + 1] = 0.0;
+            jit[a] = jitter * sf * sf;
+        }
+        CUDA_TRY(cudaMemcpyAsync(f.hyp, hk.data(), hk.size() * 8, cudaMemcpyHostToDevice, h->st));
+        CUDA_TRY(cudaMemcpyAsync(h->dJit, jit.data(), nl * 8, cudaMemcpyHostToDevice, h->st));
+        CUDA_TRY(cudaStreamSynchronize(h->st));
+    }
+    CUDA_TRY(cudaMemsetAsync(h->dInfo, 0, nl * sizeof(int), h->st));
+    CUDA_TRY(cudaEventRecord(f.ev[0], h->st));
+    int rc = launch_kbuild(h, f.hyp, h->dJit, h->dL, nl, 0);
+    if (rc) return rc;
+    rc = potrf_inv_rec(h, h->dL, f.P[0], sP, sP, h->dInfo, 0, mp, nl);
+    if (rc) return rc;
+    CUDA_TRY(cudaEventRecord(f.ev[1], h->st));
+    rc = fitc_check_info(h, "Kuu + jitter sf2 I", inf);
+    if (rc) return rc;
+    // 2. panels: Kuf -> V = Luu^-1 Kuf -> column pass -> b += Vs w, Phi += Vs Vs^T (Phi in P1)
+    {
+        const int KD = (Nx + 3) & ~3, S = ((KD >> 2) & 1) ? KD : KD + 4;
+        const int smem = (2 * KB2_TILE * S + 2 * KB2_TILE + 256) * 8;
+        CUDA_TRY(cudaFuncSetAttribute(kcross_dmma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        for (int p = 0; p < npan; ++p) {
+            const long long c0 = (long long)p * nb;
+            const int ncols = (int)std::min<long long>(nb, N - c0);
+            CUDA_TRY(cudaEventRecord(f.ev[2 + 4 * p], h->st));
+            dim3 gk((mp / KB2_TILE) * (nb / KB2_TILE), 1, nl);
+            kcross_dmma_kernel<<<gk, 256, smem, h->st>>>(h->dXT, mp, M, f.X + c0, Nq, ncols, Nx, h->dMu, h->dHyp, m,
+                                                          f.Kuf, nb, sK, nb / KB2_TILE);
+            CUDA_TRY(cudaGetLastError());
+            GemmParams q;
+            memset(&q, 0, sizeof(q));
+            q.A = f.P[0]; q.lda = mp; q.sA = sP;                        // Luu^-1: lower
+            q.B = f.Kuf; q.ldb = nb; q.sB = sK;
+            q.C = f.V; q.ldc = nb; q.sC = sK;
+            q.mt = mp / 128; q.nt = nb / 128; q.K = mp; q.alpha = 1.0; q.beta = 0.0; q.kflags = GEMM_KI_LE;
+            CUDA_TRY(cudaEventRecord(f.ev[3 + 4 * p], h->st));
+            CUDA_TRY(gemm128(h, false, q, nl));
+            CUDA_TRY(cudaEventRecord(f.ev[4 + 4 * p], h->st));
+            fitc_column_kernel<<<dim3(cpp, nl), 256, 0, h->st>>>(f.V, nb, sK, mp, ncols, h->dHyp, m, Nx, f.Y + c0, Nq,
+                                                                 f.w, nb, f.part + 2LL * p * cpp, 2 * nparts);
+            CUDA_TRY(cudaGetLastError());
+            fitc_bvec_kernel<<<dim3(mp / 8, nl), 256, 0, h->st>>>(f.V, nb, sK, nb, f.w, nb, f.b, mp);
+            CUDA_TRY(cudaGetLastError());
+            CUDA_TRY(cudaEventRecord(f.ev[5 + 4 * p], h->st));
+            memset(&q, 0, sizeof(q));
+            q.A = f.V; q.lda = nb; q.sA = sK;
+            q.B = f.V; q.ldb = nb; q.sB = sK;
+            q.C = f.P[1]; q.ldc = mp; q.sC = sP; q.Cin = f.P[1]; q.ldcin = mp; q.sCin = sP;
+            q.mt = mp / 128; q.nt = mp / 128; q.K = nb; q.alpha = 1.0; q.beta = 1.0; q.lower = 1;
+            CUDA_TRY(gemm128(h, true, q, nl));
+        }
+    }
+    CUDA_TRY(cudaEventRecord(f.ev[2 + 4 * npan], h->st));
+    // 3. A = I + Phi -> LA (P1), LA^-1 (P2)
+    fitc_add_identity_kernel<<<dim3((mp + 255) / 256, nl), 256, 0, h->st>>>(f.P[1], mp, sP, mp);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemsetAsync(h->dInfo, 0, nl * sizeof(int), h->st));
+    rc = potrf_inv_rec(h, f.P[1], f.P[2], sP, sP, h->dInfo, 0, mp, nl);
+    if (rc) return rc;
+    rc = fitc_check_info(h, "A = I + V Lambda^-1 V^T", inf);
+    if (rc) return rc;
+    // 6./7. t = LA^-1 b, NLML, alpha_s = Luu^-T (LA^-T t)   (enqueued before P1 / P2 are reused below)
+    double* t1 = f.t;
+    double* t2 = f.t + (long long)nl * mp;
+    trmv_lower_kernel<<<dim3((mp + 7) / 8, 1, nl), 256, 0, h->st>>>(f.P[2], mp, sP, f.b, mp, t1, mp, mp);
+    CUDA_TRY(cudaGetLastError());
+    fitc_nll_kernel<<<nl, 256, 0, h->st>>>(f.part, 2 * nparts, (int)nparts, f.P[1], mp, sP, t1, mp, mp, f.res);
+    CUDA_TRY(cudaGetLastError());
+    trmv_lower_T_kernel<<<dim3(mp / 32, 1, nl), 256, 0, h->st>>>(f.P[2], mp, sP, t1, mp, t2, mp, mp);
+    CUDA_TRY(cudaGetLastError());
+    trmv_lower_T_kernel<<<dim3(mp / 32, 1, nl), 256, 0, h->st>>>(f.P[0], mp, sP, t2, mp, h->dAlpha, mp, mp);
+    CUDA_TRY(cudaGetLastError());
+    // 4. X = LA^-T LA^-1 (lower, P1) through U = (LA^-1)^T (P3), the product compute_kinv uses; B' = J (I - X) J (P3)
+    for (int a = 0; a < nl; ++a) {
+        transpose_lower_kernel<<<dim3(mp / 32, mp / 32), dim3(32, 8), 0, h->st>>>(f.P[2] + a * sP, f.P[3] + a * sP, mp, mp / 32);
+        CUDA_TRY(cudaGetLastError());
+    }
+    {
+        GemmParams q;
+        memset(&q, 0, sizeof(q));
+        q.A = f.P[3]; q.lda = mp; q.sA = sP; q.B = f.P[3]; q.ldb = mp; q.sB = sP; q.C = f.P[1]; q.ldc = mp; q.sC = sP;
+        q.mt = mp / 128; q.nt = mp / 128; q.K = mp; q.alpha = 1.0; q.beta = 0.0;
+        q.kflags = GEMM_KI_GE | GEMM_KJ_GE; q.lower = 1;
+        CUDA_TRY(gemm128(h, true, q, nl));
+    }
+    const dim3 gf(mp / 32, mp / 32, nl), bf(32, 8);
+    fitc_flip_kernel<<<gf, bf, 0, h->st>>>(f.P[1], f.P[3], mp, sP, M, -1.0, 1.0);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemsetAsync(h->dInfo, 0, nl * sizeof(int), h->st));
+    rc = potrf_inv_rec(h, f.P[3], f.P[2], sP, sP, h->dInfo, 0, mp, nl);       // G (P3); G^-1 (P2) is not used
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(inf.data(), h->dInfo, nl * sizeof(int), cudaMemcpyDeviceToHost, h->st));
+    CUDA_TRY(cudaStreamSynchronize(h->st));
+    std::vector<int> shifted(nl, 0);
+    for (int a = 0; a < nl; ++a) {
+        if (!inf[a]) continue;
+        // a non-positive pivot (B is only semi-definite, e.g. duplicate inducing points give phi = 0): one retry with B + eps I
+        shifted[a] = 1;
+        fitc_flip_kernel<<<dim3(mp / 32, mp / 32, 1), bf, 0, h->st>>>(f.P[1] + a * sP, f.P[3] + a * sP, mp, sP, M, -1.0, 1.0 + FITC_B_SHIFT);
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaMemsetAsync(h->dInfo + a, 0, sizeof(int), h->st));
+        rc = potrf_inv_rec(h, f.P[3] + a * sP, f.P[2] + a * sP, sP, sP, h->dInfo + a, 0, mp, 1);
+        if (rc) return rc;
+        int i2 = 0;
+        CUDA_TRY(cudaMemcpyAsync(&i2, h->dInfo + a, sizeof(int), cudaMemcpyDeviceToHost, h->st));
+        CUDA_TRY(cudaStreamSynchronize(h->st));
+        if (i2) {
+            set_error(h, "gpmpc_fitc: output %d: B = I - A^-1 is not positive definite even with the shift %g (pivot %d)",
+                      h->a0 + a, FITC_B_SHIFT, i2 - 1);
+            return GPMPC_ERR_NOTPD;
+        }
+    }
+    // 5. S = J G^T J (P1);  R = S Luu^-1 into the L^-1 slab: lower, exact zeros above the diagonal, identity tail
+    fitc_flip_kernel<<<gf, bf, 0, h->st>>>(f.P[3], f.P[1], mp, sP, M, 1.0, 0.0);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemsetAsync(h->dLi, 0, (size_t)nl * sP * 8, h->st));
+    {
+        GemmParams q;
+        memset(&q, 0, sizeof(q));
+        q.A = f.P[1]; q.lda = mp; q.sA = sP;                            // S: lower
+        q.B = f.P[0]; q.ldb = mp; q.sB = sP;                            // Luu^-1: lower -> Bop[k][j] = 0 for k < j
+        q.C = h->dLi; q.ldc = mp; q.sC = sP;
+        q.mt = mp / 128; q.nt = mp / 128; q.K = mp; q.alpha = 1.0; q.beta = 0.0;
+        q.kflags = GEMM_KI_LE | GEMM_KJ_GE; q.lower = 1;
+        CUDA_TRY(gemm128(h, false, q, nl));
+    }
+    CUDA_TRY(cudaEventRecord(f.ev[3 + 4 * npan], h->st));
+    std::vector<double> res(nl);
+    CUDA_TRY(cudaMemcpyAsync(res.data(), f.res, nl * 8, cudaMemcpyDeviceToHost, h->st));
+    CUDA_TRY(cudaStreamSynchronize(h->st));
+    {
+        auto el = [&](int i, int j) { float ms = 0.f; cudaEventElapsedTime(&ms, f.ev[i], f.ev[j]); return (double)ms; };
+        double t[5] = {0, 0, 0, 0, 0};
+        for (int p = 0; p < npan; ++p) {
+            const int e = 2 + 4 * p;
+            t[0] += el(e, e + 1); t[1] += el(e + 1, e + 2); t[2] += el(e + 2, e + 3); t[3] += el(e + 3, e + 4);
+        }
+        t[4] = el(0, 1) + el(2 + 4 * npan, 3 + 4 * npan);
+        for (int k = 0; k < 5; ++k) h->fitc_ms[k] = t[k];
+    }
+    for (int a = 0; a < nl; ++a) {
+        if (info) info[a] = shifted[a];
+        if (nll) nll[a] = res[a];
+        h->jitter_used[a] = 0;
+    }
+    h->factorized = true; h->sparse = true; h->u_valid = false;
     return GPMPC_OK;
 }
 
@@ -735,12 +966,24 @@ extern "C" int gpmpc_nlml(gpmpc_handle_t h, int a, const double* theta, double* 
     return GPMPC_OK;
 }
 
+extern "C" int gpmpc_fitc_timings(gpmpc_handle_t h, double* ms5)
+{
+    if (!h || !ms5) return GPMPC_ERR_ARG;
+    if (!h->sparse) { set_error(h, "gpmpc_fitc_timings: no FITC build on this handle"); return GPMPC_ERR_STATE; }
+    for (int k = 0; k < 5; ++k) ms5[k] = h->fitc_ms[k];
+    return GPMPC_OK;
+}
+
 extern "C" int gpmpc_get(gpmpc_handle_t h, int what, int a, double* dst)
 {
     if (!h || !dst) return GPMPC_ERR_ARG;
     CUDA_TRY(cudaSetDevice(h->device));
     const int al = local_index(h, a);
     if (al < 0) return GPMPC_ERR_ARG;
+    if (h->sparse && h->factorized && (what == GPMPC_GET_CHOL || what == GPMPC_GET_K || what == GPMPC_GET_INVK || what == GPMPC_GET_LOGDET)) {
+        set_error(h, "gpmpc_get: selector %d has no FITC counterpart (the handle holds a sparse model: GET_ALPHA / GET_LINV)", what);
+        return GPMPC_ERR_STATE;
+    }
     if (what == GPMPC_GET_K) return gpmpc_build_K(h, a, dst);
     if (what == GPMPC_GET_ALPHA_NLML) {       // alpha of the last gpmpc_nlml(a, theta) evaluation
         CUDA_TRY(cudaMemcpyAsync(dst, h->dAlpha + (long long)al * h->Npad, h->N * 8, cudaMemcpyDeviceToHost, h->st));
@@ -769,7 +1012,15 @@ extern "C" int gpmpc_get(gpmpc_handle_t h, int what, int a, double* dst)
 extern "C" int gpmpc_set_option(gpmpc_handle_t h, const char* name, double value)
 {
     if (!h || !name) return GPMPC_ERR_ARG;
-    if (!strcmp(name, "refine")) { h->opt_refine = value != 0.0; return GPMPC_OK; }
+    if (!strcmp(name, "refine")) {
+        if (h->sparse) { set_error(h, "refine: a FITC model keeps Luu, not the factor of R, in the L slab"); return GPMPC_ERR_STATE; }
+        h->opt_refine = value != 0.0; return GPMPC_OK;
+    }
+    if (!strcmp(name, "fitc_panel")) {       // training points per FITC panel (multiple of 128)
+        const int v = (int)value;
+        if (v < 128 || v % 128 || v > 65536) { set_error(h, "fitc_panel must be a multiple of 128 in [128, 65536]"); return GPMPC_ERR_ARG; }
+        h->opt_fitc_panel = v; return GPMPC_OK;
+    }
     if (!strcmp(name, "predict_ctas")) {       // persistent grid of the predict product (0 = 2 per SM)
         const int v = (int)value;
         if (v < 0 || v > PSK_MAX_CTAS) { set_error(h, "predict_ctas must be in [0, %d]", PSK_MAX_CTAS); return GPMPC_ERR_ARG; }
@@ -1626,6 +1877,7 @@ extern "C" int gpmpc_append(gpmpc_handle_t h, const double* x_new, const double*
 {
     if (!h || !x_new || !y_new) return GPMPC_ERR_ARG;
     if (!h->factorized) { set_error(h, "gpmpc_append: call gpmpc_factorize first"); return GPMPC_ERR_STATE; }
+    if (h->sparse) { set_error(h, "gpmpc_append: the handle holds a FITC model (rebuild it with gpmpc_fitc)"); return GPMPC_ERR_STATE; }
     if (h->N >= h->Npad) { set_error(h, "gpmpc_append: capacity %d reached, refit on a new handle", h->Npad); return GPMPC_ERR_STATE; }
     CUDA_TRY(cudaSetDevice(h->device));
     int rc = ensure_predict_bufs(h, 1);

@@ -2047,3 +2047,206 @@ hess_cov_kernel(int Ny, int Nx, int method_ta, const double* __restrict__ Sigma,
         o[e * Nx + d] = s;
     }
 }
+
+// ---------------------------------------------------------------------------------------
+// FITC sparse build (gpmpc_fitc; the reference's GP.sparse, gp_class.py:682-689).  The M inducing points are the
+// handle's own points U; the N training points stream through in column panels of Nb.
+// ---------------------------------------------------------------------------------------
+// Cross-covariance panel  Kuf[:, panel] = sf2 exp(-1/2 |(u_i - x_j)/ell|^2)  (Mpad x Nb, row-major, ld = ldk): the K
+// build's scheme (centred, scaled coordinates on the handle's dMu, rank-Nx DMMA product, table exp2) on a rectangular
+// grid of 128x128 tiles, rows from U (ld ldu, M valid) and columns from the panel's X^T (ld ldf, ncols valid).  No
+// mirroring, no noise or jitter; rows >= M and columns >= ncols are exact zeros.  log2 k is clamped to log2 sf2 from
+// above everywhere (a training point that is also an inducing point has distance 0 up to rounding).
+__global__ void __launch_bounds__(256)
+kcross_dmma_kernel(const double* __restrict__ UT, int ldu, int M, const double* __restrict__ FT, long long ldf, int ncols,
+                   int Nx, const double* __restrict__ mu, const double* __restrict__ hyp, int hyp_ld,
+                   double* __restrict__ K, int ldk, long long sK, int ntj)
+{
+    extern __shared__ double sm[];
+    const int KD = (Nx + 3) & ~3;
+    const int S = ((KD >> 2) & 1) ? KD : KD + 4;
+    double* Ui = sm;                                      // [128][S] rows (inducing points)
+    double* Uj = Ui + KB2_TILE * S;                       // [128][S] columns (training points of the panel)
+    double* qi = Uj + KB2_TILE * S;
+    double* qj = qi + KB2_TILE;
+    double* T32 = qj + KB2_TILE;
+
+    const int a = blockIdx.z;
+    const double* hp = hyp + (long long)a * hyp_ld;
+    const int bi = blockIdx.x / ntj, bj = blockIdx.x - bi * ntj;
+    const int i0 = bi * KB2_TILE, j0 = bj * KB2_TILE;
+    const int tid = threadIdx.x;
+    const double sf2 = hp[Nx] * hp[Nx];
+    const double l2sf2 = log2(sf2);
+
+    __shared__ double sc[36], mus[36];
+    if (tid < S) {
+        sc[tid] = (tid < Nx) ? 1.2011224087864498 / hp[tid] : 0.0;
+        mus[tid] = (tid < Nx) ? mu[tid] : 0.0;
+    }
+    if (tid < 16) T32[tid] = c_exp2_tab[tid];
+    else if (tid < 32) T32[tid] = c_exp2_tab2[tid - 16];
+    __syncthreads();
+    {
+        const bool rowpt = tid < KB2_TILE;
+        const int l = tid & (KB2_TILE - 1);
+        double* U = rowpt ? Ui + l * S : Uj + l * S;
+        double nrm = 0.0;
+        for (int d = 0; d < S; ++d) {
+            double u = 0.0;
+            if (d < Nx) u = ((rowpt ? UT[(long long)d * ldu + i0 + l] : FT[(long long)d * ldf + j0 + l]) - mus[d]) * sc[d];
+            U[d] = u;
+            nrm = fma(u, u, nrm);
+        }
+        (rowpt ? qi : qj)[l] = fma(-0.5, nrm, 0.5 * l2sf2);
+    }
+    __syncthreads();
+
+    const int warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
+    double* Ka = K + (long long)a * sK;
+    const int nk4 = KD >> 2;
+#pragma unroll 1
+    for (int mi = 0; mi < 2; ++mi) {
+        const int rl = warp * 16 + mi * 8 + g;
+        const int row = i0 + rl;
+        const double* ua = Ui + rl * S + t;
+        const double qr = qi[rl];
+        double* drow = Ka + (long long)row * ldk + j0 + 2 * t;
+#pragma unroll 1
+        for (int ng = 0; ng < 4; ++ng) {
+            double acc[4][2];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) { acc[q][0] = 0.0; acc[q][1] = 0.0; }
+            const double* ub = Uj + (ng * 32 + g) * S + t;
+            for (int kk = 0; kk < nk4; ++kk) {
+                const double av = ua[kk * 4];
+#pragma unroll
+                for (int q = 0; q < 4; ++q) dmma884(acc[q][0], acc[q][1], av, ub[q * 8 * S + kk * 4]);
+            }
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const int cl0 = ng * 32 + q * 8;
+                const double2 qc = *reinterpret_cast<const double2*>(qj + cl0 + 2 * t);
+                double t0 = (qr + qc.x) + acc[q][0], t1 = (qr + qc.y) + acc[q][1];
+                t0 = (t0 < -1020.0) ? -1020.0 : t0;
+                t1 = (t1 < -1020.0) ? -1020.0 : t1;
+                t0 = (t0 > l2sf2) ? l2sf2 : t0;
+                t1 = (t1 > l2sf2) ? l2sf2 : t1;
+                double v0 = exp2_t2lvl(t0, T32), v1 = exp2_t2lvl(t1, T32);
+                const int col = j0 + cl0 + 2 * t;
+                if (row >= M || col >= ncols) v0 = 0.0;
+                if (row >= M || col + 1 >= ncols) v1 = 0.0;
+                *reinterpret_cast<double2*>(drow + cl0) = make_double2(v0, v1);
+            }
+        }
+    }
+}
+
+// FITC column pass over one panel of V = Luu^-1 Kuf (Mpad x Nb, ld = ld): for every column i < ncols
+//   Lambda_i = max(sf2 - |V_:i|^2, 0) + sn2       (the clamp absorbs rounding when x_i is itself an inducing point)
+//   V_:i *= Lambda_i^-1/2 (in place),  w_i = y_i Lambda_i^-1/2,  partials {sum log Lambda_i, sum y_i^2 / Lambda_i}
+// Columns >= ncols (zero in V) get w = 0 and contribute nothing.  CTA = 32 columns x 8 row groups; the row-group sums and
+// the per-CTA partials are combined in a fixed order (deterministic).  grid (Nb / 32, outputs).
+__global__ void __launch_bounds__(256)
+fitc_column_kernel(double* __restrict__ V, int ld, long long sV, int Mpad, int ncols,
+                   const double* __restrict__ hyp, int hyp_ld, int Nx, const double* __restrict__ y, long long sy,
+                   double* __restrict__ w, long long sw, double* __restrict__ part, long long spart)
+{
+    __shared__ double red[8][33];
+    __shared__ double scl[32];
+    const int lane = threadIdx.x & 31, grp = threadIdx.x >> 5, a = blockIdx.y;
+    const int col = blockIdx.x * 32 + lane;
+    double* Va = V + (long long)a * sV;
+    double s = 0.0;
+    for (int r = grp; r < Mpad; r += 8) { const double v = Va[(long long)r * ld + col]; s = fma(v, v, s); }
+    red[grp][lane] = s;
+    __syncthreads();
+    if (grp == 0) {
+        double q = 0.0;
+#pragma unroll
+        for (int k = 0; k < 8; ++k) q += red[k][lane];
+        const double* hp = hyp + (long long)a * hyp_ld;
+        const double sf2 = hp[Nx] * hp[Nx], sn2 = hp[Nx + 1] * hp[Nx + 1];
+        const bool valid = col < ncols;
+        double lam = sf2 - q;
+        lam = (lam > 0.0 ? lam : 0.0) + sn2;
+        const double is = valid ? 1.0 / sqrt(lam) : 0.0;
+        const double yv = valid ? y[(long long)a * sy + col] : 0.0;
+        scl[lane] = is;
+        w[(long long)a * sw + col] = yv * is;
+        double lp = valid ? log(lam) : 0.0, yy = valid ? yv * yv / lam : 0.0;
+        lp = warp_sum(lp); yy = warp_sum(yy);
+        if (lane == 0) {
+            part[(long long)a * spart + 2 * blockIdx.x] = lp;
+            part[(long long)a * spart + 2 * blockIdx.x + 1] = yy;
+        }
+    }
+    __syncthreads();
+    const double is = scl[lane];
+    for (int r = grp; r < Mpad; r += 8) Va[(long long)r * ld + col] *= is;
+}
+
+// b += Vs w  (b = V Lambda^-1 y accumulated panel by panel): one warp per row, lanes stride the Nb columns, fixed-order
+// warp reduction; panels are added in stream order (deterministic).  grid (Mpad / 8, outputs).
+__global__ void __launch_bounds__(256)
+fitc_bvec_kernel(const double* __restrict__ V, int ld, long long sV, int Nb, const double* __restrict__ w, long long sw,
+                 double* __restrict__ b, long long sb)
+{
+    const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31, a = blockIdx.y;
+    const double* Vr = V + (long long)a * sV + (long long)row * ld;
+    const double* wa = w + (long long)a * sw;
+    double s = 0.0;
+    for (int i = lane; i < Nb; i += 32) s = fma(Vr[i], wa[i], s);
+    s = warp_sum(s);
+    if (lane == 0) b[(long long)a * sb + row] += s;
+}
+
+// A[i][i] += 1 for i < n (A = I + Phi; Phi's padded rows are zero, so the tail becomes the identity)
+__global__ void fitc_add_identity_kernel(double* __restrict__ A, int ld, long long sA, int n)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) A[(long long)blockIdx.y * sA + (long long)i * ld + i] += 1.0;
+}
+
+// Exchange-matrix flip of the leading M x M block, lower triangle only:
+//   dst[i][j] = scale * src[M-1-j][M-1-i] + (i == j ? dadd : 0)   for j <= i < M   (reads src's lower triangle)
+// zeros above the diagonal, identity tail.  scale = -1, dadd = 1 (+ eps): J (I - X) J from X = LA^-T LA^-1 (lower);
+// scale = 1, dadd = 0: S = J G^T J from the Cholesky factor G.  grid (ld / 32, ld / 32, batch), block (32, 8).
+__global__ void fitc_flip_kernel(const double* __restrict__ src, double* __restrict__ dst, int ld, long long s, int M,
+                                 double scale, double dadd)
+{
+    const int j = blockIdx.x * 32 + threadIdx.x;
+    const double* sa = src + (long long)blockIdx.z * s;
+    double* da = dst + (long long)blockIdx.z * s;
+    for (int i = blockIdx.y * 32 + threadIdx.y; i < blockIdx.y * 32 + 32; i += 8) {
+        double v;
+        if (i < M && j < M) v = (j <= i) ? scale * sa[(long long)(M - 1 - j) * ld + (M - 1 - i)] + (i == j ? dadd : 0.0) : 0.0;
+        else v = (i == j) ? 1.0 : 0.0;
+        da[(long long)i * ld + j] = v;
+    }
+}
+
+// FITC negative log marginal likelihood per output (reference convention, no N/2 log 2 pi):
+//   1/2 (y^T Lambda^-1 y - |LA^-1 b|^2) + 1/2 (sum log Lambda_i + 2 sum log LA_ii)
+// from the column-pass partials (nparts pairs), t = LA^-1 b and LA's diagonal.  One CTA per output, fixed-order sums.
+__global__ void __launch_bounds__(256)
+fitc_nll_kernel(const double* __restrict__ part, long long spart, int nparts, const double* __restrict__ LA, int ld,
+                long long sL, const double* __restrict__ t, long long st, int n, double* __restrict__ nll)
+{
+    __shared__ double r[4][8];
+    const int a = blockIdx.x, tid = threadIdx.x;
+    const double* pa = part + (long long)a * spart;
+    const double* La = LA + (long long)a * sL;
+    const double* ta = t + (long long)a * st;
+    double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
+    for (int k = tid; k < nparts; k += 256) { s0 += pa[2 * k]; s1 += pa[2 * k + 1]; }
+    for (int i = tid; i < n; i += 256) { s2 = fma(ta[i], ta[i], s2); s3 += log(La[(long long)i * ld + i]); }
+    s0 = warp_sum(s0); s1 = warp_sum(s1); s2 = warp_sum(s2); s3 = warp_sum(s3);
+    if ((tid & 31) == 0) { r[0][tid >> 5] = s0; r[1][tid >> 5] = s1; r[2][tid >> 5] = s2; r[3][tid >> 5] = s3; }
+    __syncthreads();
+    if (tid == 0) {
+        double q[4] = {0.0, 0.0, 0.0, 0.0};
+        for (int k = 0; k < 4; ++k) for (int w8 = 0; w8 < 8; ++w8) q[k] += r[k][w8];
+        nll[a] = 0.5 * (q[1] - q[2]) + 0.5 * (q[0] + 2.0 * q[3]);
+    }
+}

@@ -42,7 +42,7 @@ class GP:
                  optimizer_opts=None, hyper=None, normalize=True, multistart=1,
                  xlb=None, xub=None, ulb=None, uub=None, meta=None,
                  optimize_nummeric=True, device=None, comm=None, engine_factory=None,
-                 prior_mean_in_predict=False):
+                 prior_mean_in_predict=False, inducing=None):
         """ Initialize and optimize GP model  (reference gp_class.py:21-75)
 
         Extra keyword arguments (not in the reference): ``device`` (CUDA ordinal,
@@ -52,6 +52,11 @@ class GP:
         never adds the prior mean m(z) back when predicting (build_gp is always called without
         meanFunc, gp_class.py:69-71; SURVEY q2).  False (default) replicates that; True adds m(z)
         to the predicted mean and d m/d z to the Jacobian / Taylor covariance.
+        ``inducing``: build a FITC sparse GP instead of the dense one (see ``sparse``): an int M (M training points
+        drawn with ``np.random.default_rng(0)``) or an (M, Nx) array of inducing points in the caller's units
+        (standardised like the test inputs).  The dense N-point model is then never created, so N can exceed what
+        the dense engine holds.  With ``hyper=None`` the hyperparameters are fitted on the M-point subset (an explicit
+        array needs ``hyper``).
         """
         X = np.array(X, dtype=np.float64).copy()
         Y = np.array(Y, dtype=np.float64).copy()
@@ -74,6 +79,7 @@ class GP:
         self.__invK = None
         self.__prior_mean_in_predict = bool(prior_mean_in_predict)
         self.__xlb = self.__xub = self.__ulb = self.__uub = None
+        self.__U = None                              # standardised inducing points of a FITC model, None when dense
 
         if meta is not None:                         # gp_class.py:42-50
             self.__meanY = np.array(meta['meanY'])
@@ -89,7 +95,24 @@ class GP:
             self.__ulb, self.__uub = np.array(ulb), np.array(uub)
 
         """ Optimize hyperparameters """
-        if hyper is None:
+        if inducing is not None:
+            self.__check_sparse_supported()
+            if hyper is None:
+                if not np.isscalar(inducing):
+                    raise ValueError('an explicit array of inducing points needs hyper (the fit uses a seeded subset)')
+                if normalize:
+                    self.__fit_scalers(X, Y, xlb, xub, ulb, uub)
+                    self.__X = self.standardize(X, self.__meanZ, self.__stdZ)
+                    self.__Y = self.standardize(Y, self.__meanY, self.__stdY)
+                self.__normalize = normalize
+                self.__mean_func = mean_func
+                idx = self.__inducing_index(inducing)
+                self.__fit_on_subset(idx, optimizer_opts, multistart)
+            else:
+                self.__hyper = np.array(hyper['hyper'], dtype=np.float64)
+                self.__set_hyper_views()
+            self.__build_sparse(inducing)
+        elif hyper is None:
             self.optimize(X=X, Y=Y, opts=optimizer_opts, mean_func=mean_func,
                           xlb=xlb, xub=xub, ulb=ulb, uub=uub,
                           multistart=multistart, normalize=normalize,
@@ -181,22 +204,12 @@ class GP:
                  multistart=1, normalize=True, warm_start=False,
                  optimize_nummeric=True):
         """reference gp_class.py:78-142"""
+        self.__refuse_sparse('optimize')
         self.__mean_func = mean_func
         self.__normalize = normalize
 
         if normalize and X is not None:              # :85-99  (population std, ddof=0)
-            self.__xlb = np.array(xlb)
-            self.__xub = np.array(xub)
-            self.__ulb = np.array(ulb)
-            self.__uub = np.array(uub)
-            self.__meanY = np.mean(Y, 0)
-            self.__stdY = np.std(Y, 0)
-            self.__meanZ = np.mean(X, 0)
-            self.__stdZ = np.std(X, 0)
-            self.__meanX = np.mean(X[:, :self.__Ny], 0)
-            self.__stdX = np.std(X[:, :self.__Ny], 0)
-            self.__meanU = np.mean(X[:, self.__Ny:], 0)
-            self.__stdU = np.std(X[:, self.__Ny:], 0)
+            self.__fit_scalers(X, Y, xlb, xub, ulb, uub)
 
         if X is not None:                            # :101-117
             X = np.array(X).copy()
@@ -221,6 +234,101 @@ class GP:
         self.__lam_x = 0
         self.__set_hyper_views()
         self.__factorize()
+
+    def __fit_scalers(self, X, Y, xlb, xub, ulb, uub):
+        self.__xlb = np.array(xlb)
+        self.__xub = np.array(xub)
+        self.__ulb = np.array(ulb)
+        self.__uub = np.array(uub)
+        self.__meanY = np.mean(Y, 0)
+        self.__stdY = np.std(Y, 0)
+        self.__meanZ = np.mean(X, 0)
+        self.__stdZ = np.std(X, 0)
+        self.__meanX = np.mean(X[:, :self.__Ny], 0)
+        self.__stdX = np.std(X[:, :self.__Ny], 0)
+        self.__meanU = np.mean(X[:, self.__Ny:], 0)
+        self.__stdU = np.std(X[:, self.__Ny:], 0)
+
+    # ------------------------------------------------------------------ FITC sparse model
+    def __check_sparse_supported(self):
+        if self.__comm.world > 1:
+            raise NotImplementedError('sparse (FITC) GPs run on one GPU; this GP spans %d ranks (build it with a '
+                                      'single-process Comm)' % self.__comm.world)
+
+    def __refuse_sparse(self, what):
+        if self.__U is not None:
+            raise NotImplementedError('%s is not available on a sparse (FITC) GP: it needs the dense N-point model '
+                                      '(build a dense GP to use it)' % what)
+
+    def __inducing_index(self, M):
+        M = int(M)
+        if not 1 <= M <= self.__N:
+            raise ValueError('the number of inducing points must be in [1, N=%d], got %d' % (self.__N, M))
+        return np.sort(np.random.default_rng(0).choice(self.__N, M, replace=False))
+
+    def __fit_on_subset(self, idx, opts, multistart):
+        """Hyperparameters of a sparse GP: the dense SLSQP fit (train_gp_b200) on the inducing subset."""
+        Xs, Ys = self.__X[idx], self.__Y[idx]
+        eng = self.__engine_factory(len(idx), self.__Nx, self.__Ny, 0, self.__Ny, self.__device)
+        try:
+            eng.set_data(Xs, Ys)
+            rows = train_gp_b200(eng, Xs, Ys, meanFunc=self.__mean_func, optimizer_opts=opts, multistart=multistart)
+        finally:
+            eng.close()
+        self.__hyper = np.array(rows, dtype=np.float64)
+        self.__lam_x = 0
+        self.__set_hyper_views()
+
+    def __build_sparse(self, inducing):
+        """Replace the engine by a FITC model on the inducing points (int M: seeded subset of the training points;
+        array: inducing points in the caller's units).  The dense engine is freed first."""
+        if np.isscalar(inducing):
+            U = self.__X[self.__inducing_index(inducing)]
+        else:
+            U = np.array(inducing, dtype=np.float64).reshape(-1, self.__Nx)
+            meanZ = getattr(self, '_GP__meanZ', None)
+            if self.__normalize and meanZ is not None:
+                U = self.standardize(U, meanZ, self.__stdZ)
+        if self.__engine is not None:
+            self.__engine.close()
+            self.__engine = None
+        Y = self.__Y
+        if self.__has_prior_mean():
+            Y = np.column_stack([self.__Y[:, a] - mean_function(self.__hyper[a], self.__X, self.__mean_func)
+                                 for a in range(self.__Ny)])
+        M = U.shape[0]
+        eng = self.__engine_factory(M, self.__Nx, self.__Ny, 0, self.__Ny, self.__device)
+        try:
+            eng.set_data(U, np.zeros((M, self.__Ny)))
+            eng.set_hyper(self.__hyper)
+            info, _ = eng.fitc(self.__X, Y, jitter=1e-6)
+        except Exception:
+            eng.close()
+            raise
+        if np.any(info):
+            print('FITC: B factor needed its retry shift (duplicate or redundant inducing points?)')
+        self.__engine = eng
+        self.__mode = 'outputs'
+        self.__U = U
+        self.__invK = None
+
+    def sparse(self, M):
+        """ Sparse Gaussian Process  (reference gp_class.py:682-689, an empty stub there): "Use Fully Independent
+        Training Conditional (FITC) to approximate the GP distribution and reduce computational complexity ...
+        Reduce the model size from N to M".
+
+        Converts this GP in place and keeps its hyperparameters.  M is an int (M training points drawn with
+        np.random.default_rng(0), sorted) or an (M, Nx) array of inducing points in the caller's units.  The dense
+        engine is freed; prediction (every method, derivatives and rollout included) then costs O(M^2) per test
+        point.  The training set is kept, but methods that need the dense model raise NotImplementedError. """
+        self.__check_sparse_supported()
+        self.__build_sparse(M)
+        self.set_method(self.__gp_method)
+
+    @property
+    def inducing(self):
+        """Standardised inducing points (M, Nx) of a sparse GP, None for a dense GP."""
+        return self.__U
 
     def validate(self, X_test, Y_test):
         """ Validate GP model with test data  (reference gp_class.py:145-190; one batched
@@ -555,6 +663,7 @@ class GP:
     def update_data_all(self, X_new, Y_new):
         """ Update training data with all new observations  (reference gp_class.py:474-550):
         append, keep the hyper-parameters, rebuild chol / alpha on the GPU. """
+        self.__refuse_sparse('update_data_all')
         X_new = np.array(X_new, dtype=np.float64).copy()
         Y_new = np.array(Y_new, dtype=np.float64).copy()
         if self.__normalize:
@@ -575,6 +684,7 @@ class GP:
         (what the reference's ``update_data``, gp_class.py:384-471, set out to do); hyper-
         parameters are kept.  Falls back to a full refactorisation (``update_data_all``) when the
         padded capacity is exhausted or an update loses positive definiteness. """
+        self.__refuse_sparse('append_data')
         X_new = np.array(X_new, dtype=np.float64).reshape(-1, self.__Nx)
         Y_new = np.array(Y_new, dtype=np.float64).reshape(-1, self.__Ny)
         Xs, Ys = X_new, Y_new
@@ -601,6 +711,7 @@ class GP:
 
     def replace_data_all(self, X_new, Y_new):
         """ Replace training data with new observations  (reference gp_class.py:553-626) """
+        self.__refuse_sparse('replace_data_all')
         X_new = np.array(X_new, dtype=np.float64).copy()
         Y_new = np.array(Y_new, dtype=np.float64).copy()
         if self.__normalize:
@@ -663,9 +774,6 @@ class GP:
         """ Get the noise variance  (gp_class.py:675-678) """
         return self.__hyper_noise_variance
 
-    def sparse(self, M):
-        """ Sparse Gaussian Process -- an empty stub in the reference too (gp_class.py:682-689) """
-
     # ------------------------------------------------------------------ factors / model I/O
     def __gather_factor(self, what):
         eng = self.__engine
@@ -675,12 +783,14 @@ class GP:
         return np.stack([m for _, m in sorted(mine, key=lambda t: t[0])], 0)
 
     def get_chol(self):
+        self.__refuse_sparse('get_chol')
         return self.__gather_factor(_lib.GET_CHOL)
 
     def get_alpha(self):
         return self.__gather_factor(_lib.GET_ALPHA)
 
     def get_invK(self):
+        self.__refuse_sparse('get_invK')
         if self.__invK is None:
             self.__invK = self.__gather_factor(_lib.GET_INVK)
         return self.__invK
@@ -715,6 +825,7 @@ class GP:
 
     def save_model(self, filename):
         """ Save model to a json file  (reference gp_class.py:729-734) """
+        self.__refuse_sparse('save_model')
         output_dict = self._GP__to_dict()
         with open(filename + ".json", "w") as outfile:
             json.dump(output_dict, outfile)
@@ -723,6 +834,7 @@ class GP:
         """ Binary side-car of save_model for large N (a 16384^2 factor is ~5 GB as JSON text):
         same fields, one compressed .npz; chol / invK are NOT stored (they are recomputed on the
         GPU at load time, as load_model does anyway). """
+        self.__refuse_sparse('save_model_npz')
         d = dict(X=self.__X, Y=self.__Y, hyper=self.__hyper, mean_func=np.array(self.__mean_func),
                  normalize=np.array(bool(self.__normalize)))
         if self.__normalize:

@@ -99,6 +99,25 @@ int gpmpc_build_K(gpmpc_handle_t h, int a, double* K_out);
  * gp_class.py:516-537). */
 int gpmpc_factorize(gpmpc_handle_t h, double jitter, int* info);
 
+/* FITC sparse model (the reference's GP.sparse, gp_class.py:682-689): the handle's own points (gpmpc_set_data, M rows)
+ * are the inducing points U; X:(N,Nx), Y:(N,Ny) host are the training set in the GP's input space, streamed through the
+ * GPU in column panels (option "fitc_panel", default 4096 points), so device memory is O(M^2 + M * panel + N (Nx+Ny)).
+ * With Kuu = k(U,U) + jitter * sf2 I (jitter e.g. 1e-6), Lambda = diag(Kff - Kfu Kuu^-1 Kuf) + sn2 I:
+ *   mean(z) = k(U,z)^T alpha_s,  var(z) = sf2 - k(U,z)^T K~^-1 k(U,z),  K~^-1 = Kuu^-1 - (Kuu + Kuf Lambda^-1 Kfu)^-1
+ * After the call the handle is factorised and sparse: the L^-1 slab holds R (lower, R^T R = K~^-1) and alpha holds
+ * alpha_s, so every predict entry point (and gp_b200_bind) evaluates the FITC prediction with the dense kernels.
+ * gpmpc_get returns alpha_s for GET_ALPHA and R for GET_LINV, GPMPC_ERR_STATE for CHOL, K, INVK and LOGDET;
+ * gpmpc_append and option "refine" return GPMPC_ERR_STATE; gpmpc_factorize turns the handle back into a dense GP on
+ * its own points.  info:(out_count,) may be NULL: 0 ok, 1 = B = I - A^-1 needed the retry shift 1e-10 I (the variance
+ * then moves by at most 1e-10 sf2).  nll:(out_count,) may be NULL: FITC negative log marginal likelihood per owned output
+ * (no N/2 log 2 pi term, as gpmpc_nlml).  GPMPC_ERR_ARG for N < 1, N > 2^30 (panel indexing is int), a zero noise
+ * level or a negative jitter; GPMPC_ERR_NOTPD (the text names the output and Kuu, A or B) when a factor fails. */
+int gpmpc_fitc(gpmpc_handle_t h, int N, const double* X, const double* Y, double jitter, int* info, double* nll);
+
+/* CUDA-event phase times (ms) of the handle's last gpmpc_fitc, summed over panels and outputs: ms5 = {Kuf build,
+ * V = Luu^-1 Kuf product, column pass + b, SYRK, M-sized factorisations and products (Kuu, A, B, R, alpha_s)}. */
+int gpmpc_fitc_timings(gpmpc_handle_t h, double* ms5);
+
 /* Negative log marginal likelihood of global output a at theta:(Nx+2,) host and
  * (grad != NULL) its analytic gradient:  NLL = 1/2 y^T alpha + 1/2 logdet K (no
  * N/2 log 2pi term), with the same jitter retry.  Replaces calc_NLL_numpy,

@@ -1,7 +1,7 @@
 """Small end-to-end pass over every kernel of the engine for compute-sanitizer
 (memcheck / racecheck / synccheck / initcheck):  K build, leaf + DMMA GEMMs (cp.async and TMA
 tensor-map feeds), alpha, NLML + gradient, the persistent stream-K predict kernel with tile
-fix-ups (several grid sizes, lower and upper mode), predict_grad, predict_hess (W passes, pair sums), EM, rank-1 append, GP.covar.
+fix-ups (several grid sizes, lower and upper mode), predict_grad, predict_hess (W passes, pair sums), EM, rank-1 append, GP.covar, the FITC build.
     compute-sanitizer --tool racecheck python tools/sanitize_run.py"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -46,4 +46,15 @@ eng.factorize()
 ok = eng.append(p['X'][0] + 0.3, p['Y'][0])
 print('append', ok, flush=True)
 eng.close()
+# FITC build: three panels of 256 points (the last one partial), M = 150 (not a multiple of 128), then predict on it
+from tests import _fitc_oracle as fo
+U = p['X'][fo.seeded_subset(N, 150)]
+sp = gp_mpc_b200.Engine(150, Nx, Ny, device=0)
+sp.set_option('fitc_panel', 256)
+sp.set_data(U, np.zeros((150, Ny))); sp.set_hyper(p['hyper'])
+info, nll = sp.fitc(p['X'], p['Y'])
+mw, vw, nw = fo.predict('direct', U, p['X'], p['Y'], p['hyper'], p['Z'])
+mean, var, _, _ = sp.predict(p['Z'], p['Sigma'], L.METHOD_TA)
+print('fitc', relinf(mean, mw), relinf(var, vw), relinf(nll, nw), flush=True)
+sp.close()
 print('done', flush=True)
